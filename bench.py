@@ -12,12 +12,19 @@ gradient (+KL slot) per minibatch; value = all ranks' env-steps / max-over-ranks
 Timing: W >= 3 warm-up epochs, then exactly K epochs, each bracketed by CUDA events on the launching stream,
 L2 flushed (256 MiB write) between epochs outside the event pairs, barrier + synchronize on both sides of the
 timed region, max over ranks.  nvidia-smi clocks are sampled during the timed region.
+
+--dump-outputs DIR (B200 arm): after the timed epochs, rank 0 writes what the last one handed its caller -- the
+per-minibatch losses, per-mini-epoch KLs and learning rate of train_epoch()'s tuple, and the model state it left --
+as DIR/<name>.npy.  Every input is seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -25,6 +32,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # a measurement writes nothing into the tree it runs from
 _STDOUT = sys.stdout
 
 WORKLOADS = {
@@ -55,7 +63,7 @@ def make_params(w, device, env_name, multi_gpu, graph=True, seed=5, mixed_precis
               'e_clip': 0.2, 'clip_value': True, 'use_smooth_clamp': True, 'bound_loss_type': 'regularisation',
               'bounds_loss_coef': 0.0, 'max_epochs': -1, 'num_actors': w['num_actors'], 'horizon_length': w['horizon'],
               'minibatch_size': w['minibatch'], 'mini_epochs': w['mini_epochs'], 'critic_coef': 2, 'print_stats': False,
-              'train_dir': '/tmp/b200_bench_runs', 'b200_cuda_graph': graph,
+              'train_dir': train_dir(), 'b200_cuda_graph': graph,
               'env_config': {'obs_dim': w['obs_dim'], 'act_dim': w['act_dim'], 'device': device, 'seed': seed}}
     if w.get('seq_length'):
         config['seq_length'] = w['seq_length']
@@ -65,6 +73,18 @@ def make_params(w, device, env_name, multi_gpu, graph=True, seed=5, mixed_precis
 
 
 CFG_OVERRIDES = {}
+TRAIN_DIR = None
+MAX_DUMP_BYTES = 64 << 20
+
+
+def train_dir():
+    """The agents' train_dir (checkpoints, summaries): a private temporary directory per process, removed at exit, so that a run
+    writes nothing into the tree and runs by different users on one machine cannot collide."""
+    global TRAIN_DIR
+    if TRAIN_DIR is None:
+        TRAIN_DIR = tempfile.mkdtemp(prefix='b200_bench_')
+        atexit.register(shutil.rmtree, TRAIN_DIR, True)
+    return TRAIN_DIR
 
 
 class ClockSampler(threading.Thread):
@@ -225,9 +245,10 @@ def build_agent(w, device, env_name, multi_gpu, graph=True, mixed_precision=True
 
 
 def timed_epochs(agent, steps, flush, world):
+    """Runs `steps` epochs; returns (ms per epoch, what the last train_epoch() returned)."""
     import torch.distributed as dist
     from rl_games_b200 import ops
-    evs = []
+    evs, result = [], None
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
@@ -237,13 +258,33 @@ def timed_epochs(agent, steps, flush, world):
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
         agent.epoch_num += 1
-        agent.train_epoch()
+        result = agent.train_epoch()
         e.record()
         evs.append((s, e))
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
-    return [s.elapsed_time(e) for s, e in evs]
+    return [s.elapsed_time(e) for s, e in evs], result
+
+
+def dump_outputs(out_dir, agent, result):
+    """Writes train_epoch()'s returned statistics (a_losses, c_losses, b_losses, entropies: one value per minibatch update; kls: one per
+    mini-epoch; last_lr) and the model state it left (model.<state_dict key>) as float32 / float64 .npy files."""
+    import numpy as np
+    _, _, _, _, a_losses, c_losses, b_losses, entropies, kls, last_lr, _ = result
+    arrays = {k: torch.stack([torch.as_tensor(x, dtype=torch.float32) for x in v]).numpy()
+              for k, v in (('a_losses', a_losses), ('c_losses', c_losses), ('b_losses', b_losses), ('entropies', entropies), ('kls', kls))
+              if len(v)}
+    arrays['last_lr'] = np.array([last_lr], dtype=np.float64)
+    for k, v in agent.model.state_dict().items():
+        v = v.detach().cpu()          # fp64 normaliser moments and integer counts stay exact in float64
+        arrays['model.' + k] = (v.double() if v.dtype == torch.float64 or not v.is_floating_point() else v.float()).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > MAX_DUMP_BYTES:
+        raise SystemExit(f'bench.py: --dump-outputs would write {total} bytes (limit {MAX_DUMP_BYTES})')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
 
 
 def kernel_breakdown(agent):
@@ -343,8 +384,10 @@ def b200_arm(args, w):
     sampler = ClockSampler(local_rank)
     sampler.start()
     time.sleep(0.3)
-    ms = timed_epochs(agent, args.steps, flush, world)
+    ms, result = timed_epochs(agent, args.steps, flush, world)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, agent, result)
     total_ms = torch.tensor([sum(ms)], dtype=torch.float64, device=device)
     if multi:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -424,7 +467,7 @@ def b200_arm(args, w):
             agent._repack()
         timed_epochs(agent, 3, flush, world)
         k5 = max(3, min(args.steps, 10))
-        ms5 = timed_epochs(agent, k5, flush, world)
+        ms5, _ = timed_epochs(agent, k5, flush, world)
         t5 = torch.tensor([sum(ms5)], dtype=torch.float64, device=device)
         if multi:
             dist.all_reduce(t5, op=dist.ReduceOp.MAX)
@@ -444,6 +487,7 @@ def b200_arm(args, w):
         dist.barrier()
         sys.stderr.flush()
         _STDOUT.flush()
+        shutil.rmtree(train_dir(), ignore_errors=True)      # os._exit skips the atexit removal
         os._exit(0)
 
 
@@ -482,7 +526,13 @@ def main():
     ap.add_argument('--skip-e2e', action='store_true')
     ap.add_argument('--skip-cpu', action='store_true')
     ap.add_argument('--skip-secondary', action='store_true', help='do not append the c5 block to the c2 line')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed epoch returned and the model state it left as DIR/<name>.npy (B200 arm)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to the B200 arm')
     w = WORKLOADS[args.workload]
     import ast
     for kv in args.cfg:

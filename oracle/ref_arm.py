@@ -14,11 +14,13 @@ The UNMODIFIED reference (Denys88/rl_games) as the CPU arm of bench.py (`--impl 
   `Runner.algo_factory` with the env injected via config['env_info'] / config['vec_env'] (a2c_common.py:236-241),
   device cpu, mixed_precision False, torch_compile False, compute_gae -> _pytorch_gae (gae_kernel.py:62-79, :139).
 """
+import atexit
 import hashlib
 import json
 import os
 import shutil
 import sys
+import tempfile
 import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -26,6 +28,7 @@ ROOT = os.path.dirname(HERE)
 REF_SRC = '/root/reference'
 REF_DST = os.path.join(HERE, '_ref')
 STUBS = os.path.join(ROOT, 'tests', 'golden', '_stubs')
+_TRAIN_DIR = None
 
 
 def _tree_digest(path):
@@ -127,6 +130,15 @@ class SyntheticVecEnvCPU:
         pass
 
 
+def _train_dir():
+    """The reference agents' train_dir: private to this process and removed at exit, so runs by different users cannot collide."""
+    global _TRAIN_DIR
+    if _TRAIN_DIR is None:
+        _TRAIN_DIR = tempfile.mkdtemp(prefix='b200_refarm_')
+        atexit.register(shutil.rmtree, _TRAIN_DIR, True)
+    return _TRAIN_DIR
+
+
 def make_params(w, num_actors, minibatch, mini_epochs=None):
     """c2 / c5 hyper-parameters (rl_games/configs/mujoco/ant_envpool.yaml:28-56), the same dict bench.py gives the B200 arm."""
     network = {'name': 'actor_critic', 'separate': False,
@@ -142,7 +154,7 @@ def make_params(w, num_actors, minibatch, mini_epochs=None):
               'e_clip': 0.2, 'clip_value': True, 'use_smooth_clamp': True, 'bound_loss_type': 'regularisation',
               'bounds_loss_coef': 0.0, 'max_epochs': -1, 'num_actors': num_actors, 'horizon_length': w['horizon'],
               'minibatch_size': minibatch, 'mini_epochs': mini_epochs or w['mini_epochs'], 'critic_coef': 2, 'save_frequency': 0,
-              'save_best_after': 10 ** 9, 'print_stats': False, 'train_dir': '/tmp/b200_refarm_runs'}
+              'save_best_after': 10 ** 9, 'print_stats': False, 'train_dir': _train_dir()}
     if w.get('seq_length'):
         config['seq_length'] = w['seq_length']
     return {'seed': 5, 'torch_threads': 0, 'algo': {'name': 'a2c_continuous'}, 'model': {'name': 'continuous_a2c_logstd'},

@@ -8,6 +8,7 @@ weights after 2 epochs (8-16 Adam steps): atol 2e-5 (Adam divides by sqrt(v): ti
 amplify 1e-7 differences); lr sequence and running-stat counts: exact.
 """
 import os
+import tempfile
 
 import numpy as np
 import pytest
@@ -18,6 +19,7 @@ from oracle import ppo_oracle as O
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(__file__), 'golden')
 DEV = 'cuda:0'
+RUNS = tempfile.TemporaryDirectory(prefix='b200_test_runs_')      # the agents' train_dir: private to this process, removed at exit
 
 
 class TapeEnvGPU:
@@ -67,7 +69,7 @@ def make_agent(cfg_over, N, H, D, A, units, mb, env, init_state, rnn_units=0, rn
               'lr_schedule': 'adaptive', 'kl_threshold': 0.008, 'grad_norm': 1.0, 'entropy_coef': 0.0, 'truncate_grads': True,
               'e_clip': 0.2, 'clip_value': True, 'use_smooth_clamp': True, 'bound_loss_type': 'regularisation',
               'bounds_loss_coef': 0.0, 'max_epochs': 100, 'num_actors': N, 'horizon_length': H, 'minibatch_size': mb,
-              'mini_epochs': 4, 'critic_coef': 2, 'print_stats': False, 'train_dir': '/tmp/b200_parity_runs'}
+              'mini_epochs': 4, 'critic_coef': 2, 'print_stats': False, 'train_dir': RUNS.name}
     config.update(cfg_over)
     config['env_info'] = env.get_env_info()
     config['vec_env'] = env
@@ -320,7 +322,7 @@ def test_synthetic_env_training_runs_and_graph_replay_is_consistent():
                              'grad_norm': 1.0, 'entropy_coef': 0.0, 'truncate_grads': True, 'e_clip': 0.2, 'clip_value': True,
                              'use_smooth_clamp': True, 'bound_loss_type': 'regularisation', 'bounds_loss_coef': 0.0,
                              'num_actors': 1024, 'horizon_length': 16, 'minibatch_size': 4096, 'mini_epochs': 2,
-                             'critic_coef': 2, 'print_stats': False, 'train_dir': '/tmp/b200_parity_runs',
+                             'critic_coef': 2, 'print_stats': False, 'train_dir': RUNS.name,
                              'mixed_precision': False, 'b200_cuda_graph': graph,
                              'env_config': {'obs_dim': 60, 'act_dim': 8, 'device': DEV}}}
         r = Runner()

@@ -53,13 +53,13 @@ def _init_rank(rank, world, port):
     torch.device = _Dev
 
 
-def _worker(rank, world, port, ret, name='agent_masked.pt', extra=None):
+def _worker(rank, world, port, ret, runs, name='agent_masked.pt', extra=None):
     _init_rank(rank, world, port)
     import test_agent_host_cpu as H
     from oracle import ppo_oracle as O
     from test_oracle_vs_golden import _oracle_from_golden
     g = _rank_tapes(torch.load(os.path.join(GOLDEN, name), weights_only=False), rank)
-    agent = H._build(_Patch(), '/tmp/b200_multirank_%d' % rank, g, H._Env(g),
+    agent = H._build(_Patch(), os.path.join(runs, str(rank)), g, H._Env(g),
                      over={'multi_gpu': True, 'b200_fused_allreduce': False, 'print_stats': False, **(extra or {})})
     assert agent.multi_gpu and agent.world_size == 2 and agent.global_rank == rank and not agent.fused_allreduce
     ar = lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM)      # noqa: E731
@@ -96,11 +96,11 @@ def _worker(rank, world, port, ret, name='agent_masked.pt', extra=None):
                                         ('agent_minsigma.pt', None),            # sigma floor: the chained log-std gradient is what gets averaged
                                         ('agent_separate.pt', None)],           # separate trunks: the masked gradient is what gets averaged
                          ids=['per-minibatch schedule', 'per-mini-epoch schedule', 'min_sigma', 'separate trunks'])
-def test_two_rank_agent_matches_oracle_and_ranks_stay_identical(name, extra):
+def test_two_rank_agent_matches_oracle_and_ranks_stay_identical(name, extra, tmp_path):
     world, port = 2, 29500 + (os.getpid() + len(name)) % 400
     mgr = mp.Manager()
     ret = mgr.dict()
-    mp.spawn(_worker, args=(world, port, ret, name, extra), nprocs=world, join=True)
+    mp.spawn(_worker, args=(world, port, ret, str(tmp_path), name, extra), nprocs=world, join=True)
     g = torch.load(os.path.join(GOLDEN, name), weights_only=False)
     for ep in range(len(g['epochs_out'])):
         (p0, lr0, c0, m0, r0), (p1, lr1, c1, m1, r1) = ret[0][ep], ret[1][ep]
@@ -113,7 +113,7 @@ def test_two_rank_agent_matches_oracle_and_ranks_stay_identical(name, extra):
     assert not torch.allclose(ret[0][-1][0][off:off + w0.numel()], w0, rtol=1e-3, atol=1e-5)
 
 
-def _worker_cv(rank, world, port, ret):
+def _worker_cv(rank, world, port, ret, runs):
     """central value (gated path): the critic has its OWN per-minibatch gradient exchange (central_value.py:322-337) and its normalisers
     join the pooled stats sync (a2c_common.py:753-765)"""
     _init_rank(rank, world, port)
@@ -124,7 +124,7 @@ def _worker_cv(rank, world, port, ret):
     if rank:
         g['state_tape'] = torch.roll(torch.flip(g['state_tape'], dims=[1]), shifts=3, dims=0).contiguous() * 0.75 - 0.1
         g['noise'] = torch.flip(torch.stack(list(g['noise'])), dims=[2]).contiguous()
-    agent = HC._build_cv(_Patch(), '/tmp/b200_multirank_cv_%d' % rank, g,
+    agent = HC._build_cv(_Patch(), os.path.join(runs, str(rank)), g,
                          over={'multi_gpu': True, 'b200_fused_allreduce': False, 'print_stats': False})
     cv = agent.central_value_net
     assert agent.multi_gpu and cv.multi_gpu and cv.world_size == 2
@@ -159,16 +159,16 @@ def _worker_cv(rank, world, port, ret):
     dist.destroy_process_group()
 
 
-def test_two_rank_central_value_agent_matches_oracle_and_ranks_stay_identical():
+def test_two_rank_central_value_agent_matches_oracle_and_ranks_stay_identical(tmp_path):
     world, port = 2, 29900 + os.getpid() % 90
     mgr = mp.Manager()
     ret = mgr.dict()
-    mp.spawn(_worker_cv, args=(world, port, ret), nprocs=world, join=True)
+    mp.spawn(_worker_cv, args=(world, port, ret, str(tmp_path)), nprocs=world, join=True)
     for (p0, c0, m0, n0), (p1, c1, m1, n1) in zip(ret[0], ret[1]):
         assert torch.equal(p0, p1) and torch.equal(c0, c1) and torch.equal(m0, m1) and n0 == n1
 
 
-def _worker_discrete(rank, world, port, ret):
+def _worker_discrete(rank, world, port, ret, runs):
     """discrete PPO (gated path): NCCL-style flat-gradient all-reduce in front of the Adam kernel, rank-mean KL for the per-mini-epoch
     scheduler (a2c_common.py:1272-1274), pooled normaliser sync"""
     _init_rank(rank, world, port)
@@ -181,7 +181,7 @@ def _worker_discrete(rank, world, port, ret):
         for k in ('obs_tape', 'done_tape', 'timeout_tape', 'mask_tape'):
             g[k] = torch.roll(torch.flip(g[k], dims=[1]), shifts=2, dims=0).contiguous()
         g['u'] = torch.flip(g['u'], dims=[-1]).contiguous()
-    agent = HD._build(_Patch(), '/tmp/b200_multirank_disc_%d' % rank, g, over={'multi_gpu': True, 'print_stats': False})
+    agent = HD._build(_Patch(), os.path.join(runs, str(rank)), g, over={'multi_gpu': True, 'print_stats': False})
     assert agent.multi_gpu and agent.world_size == 2 and agent.global_rank == rank
     ar = lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM)      # noqa: E731
     orc = _discrete_oracle_from_golden(g)
@@ -207,10 +207,10 @@ def _worker_discrete(rank, world, port, ret):
     dist.destroy_process_group()
 
 
-def test_two_rank_discrete_agent_matches_oracle_and_ranks_stay_identical():
+def test_two_rank_discrete_agent_matches_oracle_and_ranks_stay_identical(tmp_path):
     world, port = 2, 30100 + os.getpid() % 90
     mgr = mp.Manager()
     ret = mgr.dict()
-    mp.spawn(_worker_discrete, args=(world, port, ret), nprocs=world, join=True)
+    mp.spawn(_worker_discrete, args=(world, port, ret, str(tmp_path)), nprocs=world, join=True)
     for (p0, lr0, a0), (p1, lr1, a1) in zip(ret[0], ret[1]):
         assert torch.equal(p0, p1) and lr0 == lr1 and not torch.equal(a0, a1)

@@ -1,6 +1,7 @@
 """Central value (asymmetric critic) on the GPU (rl_games_b200/agent_cv.py, csrc/critic.cu); first green on a B200 in round 2.
 The host logic and the kernel's row arithmetic are also checked on CPU (tests/test_agent_cv_host_cpu.py, tests/test_critic_rows_cpu.py)."""
 import os
+import tempfile
 
 import numpy as np
 import pytest
@@ -11,6 +12,7 @@ from oracle import ppo_oracle as O
 pytestmark = [pytest.mark.gpu]
 DEV = 'cuda:0'
 GOLDEN = os.path.join(os.path.dirname(__file__), 'golden')
+RUNS = tempfile.TemporaryDirectory(prefix='b200_test_runs_')      # the agents' train_dir: private to this process, removed at exit
 
 
 @pytest.mark.parametrize('masked', [False, True])
@@ -84,7 +86,7 @@ def test_central_value_agent_matches_reference_golden(graph):
                          'mlp': {'units': g['cv_units'], 'activation': 'elu', 'initializer': {'name': 'default'}}}
     config = {k: v for k, v in cfgk.items() if k not in ('device', 'torch_compile')}
     config.update({'device': DEV, 'env_info': env.get_env_info(), 'vec_env': env, 'reward_shaper': {'scale_value': 1.0},
-                   'mixed_precision': False, 'b200_cuda_graph': graph, 'train_dir': '/tmp/b200_parity_runs',
+                   'mixed_precision': False, 'b200_cuda_graph': graph, 'train_dir': RUNS.name,
                    'lr_schedule': cfgk.get('lr_schedule', None), 'central_value_config': cv_cfg})
     network = {'name': 'actor_critic', 'separate': False,
                'space': {'continuous': {'mu_activation': 'None', 'sigma_activation': 'None', 'mu_init': {'name': 'default'},

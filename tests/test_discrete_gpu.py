@@ -2,6 +2,7 @@
 first green on a B200 in round 2.  The oracle side (oracle/ppo_discrete_oracle.py) is pinned to the real reference by
 tests/test_oracle_vs_golden.py, which runs on CPU."""
 import os
+import tempfile
 
 import numpy as np
 import pytest
@@ -12,6 +13,7 @@ from oracle import ppo_discrete_oracle as DO
 pytestmark = [pytest.mark.gpu]
 DEV = 'cuda:0'
 GOLDEN = os.path.join(os.path.dirname(__file__), 'golden')
+RUNS = tempfile.TemporaryDirectory(prefix='b200_test_runs_')      # the agents' train_dir: private to this process, removed at exit
 
 
 @pytest.mark.parametrize('masked,fused', [(False, True), (True, True), (True, False)])
@@ -132,7 +134,7 @@ def test_discrete_agent_matches_reference_golden(name):
     env = DiscreteTapeEnvGPU(g)
     config = {k: v for k, v in cfgk.items() if k not in ('device', 'torch_compile')}
     config.update({'device': DEV, 'env_info': env.get_env_info(), 'vec_env': env, 'reward_shaper': {'scale_value': 0.1},
-                   'train_dir': '/tmp/b200_parity_runs', 'lr_schedule': cfgk.get('lr_schedule', None)})
+                   'train_dir': RUNS.name, 'lr_schedule': cfgk.get('lr_schedule', None)})
     multi = isinstance(g['K'], (list, tuple))
     network = {'name': 'actor_critic', 'separate': g['separate'], 'space': {'multi_discrete' if multi else 'discrete': None},
                'mlp': {'units': g['units'], 'activation': 'relu', 'initializer': {'name': 'default'}}}

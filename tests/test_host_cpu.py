@@ -78,22 +78,22 @@ def _params(**over):
               'normalize_value': True, 'normalize_advantage': True, 'gamma': 0.99, 'tau': 0.95, 'learning_rate': 3e-4,
               'lr_schedule': 'adaptive', 'kl_threshold': 0.008, 'grad_norm': 1.0, 'entropy_coef': 0.0, 'e_clip': 0.2, 'clip_value': True,
               'num_actors': 8, 'horizon_length': 8, 'minibatch_size': 32, 'mini_epochs': 2, 'critic_coef': 2,
-              'train_dir': '/tmp/b200_cpu_tests', 'env_info': {'observation_space': Box(-1, 1, (6,)), 'action_space': Box(-1, 1, (3,))}}
+              'env_info': {'observation_space': Box(-1, 1, (6,)), 'action_space': Box(-1, 1, (3,))}}
     config.update(over)
     return {'seed': 1, 'algo': {'name': 'a2c_continuous'}, 'model': {'name': 'continuous_a2c_logstd'}, 'network': network, 'config': config}
 
 
-def test_agent_has_no_cpu_fallback_and_mirrors_config_errors():
+def test_agent_has_no_cpu_fallback_and_mirrors_config_errors(tmp_path):
     from rl_games_b200.runner import Runner
     r = Runner()
-    r.load({'params': _params()})
+    r.load({'params': _params(train_dir=str(tmp_path))})
     assert r.algo_name == 'a2c_continuous' and r.seed == 1
     with pytest.raises(RuntimeError, match='no CPU fallback'):
         r.algo_factory.create(r.algo_name, base_name='x', params=r.params)
     with pytest.raises(ValueError):
         r.algo_factory.create('sac', base_name='x', params=r.params)            # ObjectFactory: unknown name -> ValueError(name)
     r2 = Runner()
-    r2.load({'params': _params(multi_gpu_sync_stats_mode='bogus')})
+    r2.load({'params': _params(train_dir=str(tmp_path), multi_gpu_sync_stats_mode='bogus')})
     with pytest.raises(ValueError, match='multi_gpu_sync_stats_mode'):             # a2c_common.py:99-103
         r2.algo_factory.create(r2.algo_name, base_name='x', params=r2.params)
 

@@ -14,7 +14,7 @@ import pytest
 import torch
 
 from oracle import ppo_oracle as O
-from tests.test_agent_gpu import DEV, GOLDEN, _check_epoch, make_agent
+from tests.test_agent_gpu import DEV, GOLDEN, RUNS, _check_epoch, make_agent
 
 pytestmark = pytest.mark.gpu
 
@@ -135,7 +135,7 @@ def test_critic_group_feeds_the_central_value_net_like_the_reference_golden_run(
                          'mlp': {'units': g['cv_units'], 'activation': 'elu', 'initializer': {'name': 'default'}}}
     config = {k: v for k, v in cfgk.items() if k not in ('device', 'torch_compile')}
     config.update({'device': DEV, 'env_info': info, 'vec_env': env, 'reward_shaper': {'scale_value': 1.0}, 'mixed_precision': False,
-                   'b200_cuda_graph': graph, 'train_dir': '/tmp/b200_parity_runs', 'lr_schedule': cfgk.get('lr_schedule', None),
+                   'b200_cuda_graph': graph, 'train_dir': RUNS.name, 'lr_schedule': cfgk.get('lr_schedule', None),
                    'central_value_config': cv_cfg, 'algo_observer': 'isaac'})
     network = {'name': 'actor_critic', 'separate': False,
                'space': {'continuous': {'mu_activation': 'None', 'sigma_activation': 'None', 'mu_init': {'name': 'default'},

@@ -34,7 +34,7 @@ def main():
         agent.obs = agent.env_reset()
         dist.broadcast(agent.model.flat, 0)
         agent._repack()
-        ts = bench.timed_epochs(agent, 6, None, world)
+        ts, _ = bench.timed_epochs(agent, 6, None, world)
         flat = torch.cat([agent.model.flat, agent.model.exp_avg, agent.model.exp_avg_sq, agent.opt_state.float(),
                           agent.model.running_mean_std.running_mean.float(), agent.model.running_mean_std.running_var.float(),
                           agent.model.value_mean_std.running_mean.float()])
