@@ -434,7 +434,9 @@ int b200rl_bump_u64(uint64_t* p, void* stream);
  * own -- the training forward / backward calls launch them internally, the rollout forward needs `l1_scratch`, a tiled bf16
  * buffer of n_tiles(N_rows) * tile_bytes[0]; xtile must be NULL).  0 = unsupported.  Weights are consumed from ONE packed bf16 copy (b200rl_tc_pack_weights) that
  * serves the forward (K-major view) and the dgrad (MN-major view).  act1/act2/act3/dhead/delta1/delta2 are
- * opaque tiled bf16 buffers: n_tiles(M) = ceil(M/128) tiles of b200rl_tc_tile_bytes() bytes each.
+ * opaque tiled bf16 buffers: n_tiles(M) = ceil(M/128) tiles of b200rl_tc_tile_bytes() bytes each.  They, xtile and l1_scratch need no
+ * initialisation: what they hold before the kernel that fills them runs (NaN included) reaches no result -- padded rows, padded units
+ * and the d_head columns past the last action are written as zeros.
  *   fwd_train : trunk + heads + PPO loss fwd/bwd (same semantics / partial format as b200rl_ppo_head_loss_f32,
  *               finalise with b200rl_ppo_loss_finalize)
  *   fwd_rollout: trunk + heads + sample/neglogp/denorm-value epilogue (same semantics as b200rl_policy_head_sample_f32)

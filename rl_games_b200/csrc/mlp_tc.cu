@@ -683,9 +683,16 @@ __global__ void __launch_bounds__(FWD_THREADS, 1) mlp_fwd_tc_kernel(const FwdArg
                 }
                 *reinterpret_cast<float4*>(sPart + (row * 4 + h) * 4) = make_float4(sz2, kl, bl, 0.f);
             }
+            uint8_t* gd = p.dhead + (size_t)tile * N::DH_BYTES;
+            if (live && h >= 2 && p.A + 1 < 8 * (h - 1)) {
+                // d_head columns past the last action: the backward MMAs contract over all AP columns of the tile, and a zero weight row
+                // cancels stale finite data but not NaN / Inf left in a buffer that was never initialised.  One 16-byte store zeroes
+                // each 8-column chunk that holds such columns (h == 2: columns 0-7, h == 3: 8-15); the live columns of the chunk are
+                // stored over it after the barrier.
+                *reinterpret_cast<uint4*>(gd + tile_off(row, h - 2, 2048u, 128u)) = make_uint4(0, 0, 0, 0);
+            }
             __syncthreads();
             TSTAMP();   // loss phase A done
-            uint8_t* gd = p.dhead + (size_t)tile * N::DH_BYTES;
             if (live) {
                 float sz2 = 0.f, kl = 0.f, bl = 0.f;
 #pragma unroll

@@ -375,8 +375,14 @@ def test_bf16_tcgen05_agent_other_geometries_and_activations_track_fp32_agent(D,
     _bf16_vs_fp32_agents(D, {}, units=units, activation=activation)
 
 
-def _bf16_vs_fp32_agents(D, extra, units=(256, 128, 64), activation='elu'):
-    N, H, A, mb = 512, 8, 8, 2048
+def test_bf16_tcgen05_agent_with_six_actions_tracks_fp32_agent():
+    """HalfCheetah / Walker2d widths (obs 17, 6 actions) on [128, 64, 32] (configs/mujoco/halfcheetah.yaml): the tcgen05 heads at an
+    action width that is not a multiple of 4, through whole training epochs"""
+    _bf16_vs_fp32_agents(17, {}, units=[128, 64, 32], A=6)
+
+
+def _bf16_vs_fp32_agents(D, extra, units=(256, 128, 64), activation='elu', A=8):
+    N, H, mb = 512, 8, 2048
     units = list(units)
     obs_tape, done_tape, tout_tape = O.make_tapes(H + 1, N, D, seed=21)
     params = O.init_params(D, units, A, seed=4)
