@@ -287,6 +287,24 @@ int b200rl_value_loss_f32(const float* values, int value_ld, const float* old_va
                           const float* inv_count_dev, float* d_value, int dv_ld, double* partials, int max_partials,
                           int* n_blocks_out_host, void* stream);
 
+/* Fused value head of the tensor-core critic (mixed_precision: True in central_value_config).
+ *  b200rl_value_head_loss_f32 (training): a_last [M, Hl] (output of act_last), W_v [Hl], b_v [1], all fp32.
+ *    v = W_v . a_last + b_v in fp32, then b200rl_value_loss_f32's loss, weights, chunk mapping and partial rows (one per 256 rows:
+ *    {w*loss, mask, w, 0...}); d_alast [M, Hl] = dL/dv * W_v * act'(a_last); the head gradient goes into the split-partial arena
+ *    (dW_part + s*split_stride [Hl], db_part + s*split_stride [1] for s < n_splits; sum with b200rl_reduce_splits_f32).  Optional
+ *    value_out [M] receives v.  Deterministic (fixed-order sums, no atomics).  Hl <= B200RL_VALUE_HEAD_MAX_HL (else
+ *    B200RL_EUNSUPPORTED).  Outputs need no initialisation.
+ *  b200rl_value_head_fwd_f32 (rollout): values [N] = v of each row, de-normalised as b200rl_normalize_f32(denorm = 1, eps = 1e-5)
+ *    when normalize_value; the dot product has the training kernel's summation order. */
+#define B200RL_VALUE_HEAD_MAX_HL 4096
+int b200rl_value_head_loss_f32(const float* a_last, int Hl, const float* W_v, const float* b_v, const float* old_values_n,
+                               const float* returns_n, const float* mask, int rows_per_chunk, int64_t chunk_stride, int M,
+                               float e_clip, int clip_value, const float* inv_count_dev, int act_last, float* d_alast,
+                               float* value_out, float* dW_part, float* db_part, int64_t split_stride, int n_splits,
+                               double* partials, int max_partials, int* n_blocks_out_host, void* stream);
+int b200rl_value_head_fwd_f32(const float* a_last, int Hl, const float* W_v, const float* b_v, const double* vms_mean,
+                              const double* vms_var, int normalize_value, float* values, int N, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Optimiser step.  Replaces a2c_common.py:493-514 (trancate_gradients_and_step: /world_size,
  * clip_grad_norm_, optimizer.step) + torch.optim.Adam(eps=1e-8, weight_decay, fused=True)

@@ -13,8 +13,16 @@ on CPU against the same golden vectors with torch stand-ins for the kernels (``t
     GAE use them; the agent's value normaliser IS the critic's (a2c_continuous.py:72-73);
   * the critic trains (own minibatching, own Adam, own obs normaliser re-armed on every minibatch) before the actor's mini-epochs;
   * the actor keeps its own value head and value loss (``use_experimental_cv`` defaults to True in the reference).
-Scope of this first edition: one GPU, MLP critic, fp32 kernels for the critic, no whole-epoch CUDA graph (the update-phase graph of the
-actor still works), identity / linear critic LR schedule.
+Precision is the critic's own key, ``central_value_config['mixed_precision']`` (central_value.py:24), never the agent's:
+  * True: every trunk layer runs on the layer-wise tcgen05 GEMMs (``gemm_tc.cu``: bf16 operands from a bf16 twin of the critic's arena,
+    fp32 accumulate), in training and in the rollout; the 1-wide value head is one fused fp32 kernel (``csrc/critic.cu``
+    value_head_loss / value_head_fwd).  Rollout and last values come from the same kernels as training, so old and re-evaluated values
+    share arithmetic (DESIGN.md §2, §8).  The twin is refreshed after every critic optimiser step and every weight load;
+  * False: the fp32 CUDA-core kernels;
+  * absent: the fp32 kernels, with a printed note.
+``central_value_net.gemm_tc`` records the result.  The tensor-core critic's host logic is checked on CPU (``tests/test_cv_tensor_cores_cpu.py``);
+its GPU tests (``tests/test_cv_tensor_cores_gpu.py``) have not yet run on hardware.
+Scope: MLP critic, no whole-epoch CUDA graph (the update-phase graph of the actor still works), identity / linear critic LR schedule.
 """
 from collections import OrderedDict
 
@@ -76,6 +84,10 @@ class CentralValueNet:
         self.truncate_grads, self.grad_norm = bool(cv_config.get('truncate_grads', False)), float(cv_config.get('grad_norm', 1))
         self.weight_decay = float(cv_config.get('weight_decay', 0.0))
         self.freeze = bool(cv_config.get('freeze_critic', False))
+        # precision (central_value.py:24): the critic's own key, never the agent's.  True -> trunk on the layer-wise tcgen05 GEMMs
+        # (bf16 operands, fp32 accumulate) and the fused fp32 value head; False or absent -> the fp32 CUDA-core kernels
+        self.precision_set = 'mixed_precision' in cv_config
+        self.gemm_tc = bool(cv_config.get('mixed_precision', False))
         self.scheduler = (LinearScheduler(self.lr, max_steps=max_epochs, apply_to_entropy=False, start_entropy_coef=0)
                           if cv_config.get('lr_schedule') == 'linear' else IdentityScheduler())        # central_value.py:55-62
         self.epoch_num = self.frame = 0
@@ -84,6 +96,9 @@ class CentralValueNet:
             sizes += [(f'W{i}', (u, ins)), (f'b{i}', (u,))]
             ins = u
         self.Hl = ins
+        if self.gemm_tc and self.Hl > ops.VALUE_HEAD_MAX_HL:
+            raise NotImplementedError(f'central value mixed_precision: the fused value head takes a last layer of at most '
+                                      f'{ops.VALUE_HEAD_MAX_HL} units (got {self.Hl})')
         sizes += [('W_v', (1, ins)), ('b_v', (1,))]
         self.layout, off = OrderedDict(), 0
         for n, shp in sizes:
@@ -106,7 +121,8 @@ class CentralValueNet:
         self.t_act = [f(mb, u) for u in self.units]
         self.d_act = [f(mb, u) for u in self.units]
         self.r_val, self.t_val, self.d_val = f(self.N, 1), f(mb, 1), f(mb, 1)
-        self.n_splits = max(1, min(64, mb // 256))
+        # split rows of the weight gradients: the tensor-core GEMMs are sized like the actor's layer-wise path (agent.py)
+        self.n_splits = max(1, min(16, mb // 512)) if self.gemm_tc else max(1, min(64, mb // 256))
         self.part = f(self.n_splits, off)
         self.grad = f(off)
         self.loss_partials = torch.zeros((mb + 255) // 256, 8, dtype=torch.float64, device=dev)
@@ -119,6 +135,9 @@ class CentralValueNet:
         self.opt_cfg = ops.OptCfg(0.9, 0.999, 1e-8, self.weight_decay, self.grad_norm, 0.0, 1e-6, 1e-2, 1.5,
                                   1.0 / (self.world_size if self.multi_gpu else 1), int(self.truncate_grads), 0)
         self.last_losses = []
+        if self.gemm_tc:
+            self.wbf = torch.empty(off, dtype=torch.bfloat16, device=dev)      # bf16 twin of the arena: the GEMMs' weight operands
+            self.refresh_twin()
 
     def view(self, name, arena=None):
         o, shp = self.layout[name]
@@ -162,19 +181,47 @@ class CentralValueNet:
                 self.value_mean_std.load_state_dict(sd, 'value_mean_std.')
             if self.normalize_input and 'running_mean_std.running_mean' in sd:
                 self.running_mean_std.load_state_dict(sd, 'running_mean_std.')
+        self.refresh_twin()
+
+    def refresh_twin(self):
+        """the tensor-core GEMMs read the bf16 twin of the arena: refreshed after every optimiser step and every weight load (a stale
+        twin gives plausible values from the old weights)"""
+        if self.gemm_tc:
+            ops.cast_bf16(self.flat, self.wbf)
+
+    # layer GEMMs of the selected precision (looked up at call time: the ops may be replaced after construction)
+    def _lin_fwd(self, *a, **k):
+        if self.gemm_tc:
+            ops.linear_fwd_tc(*a, bf16_arena=(self.flat, self.wbf), **k)
+        else:
+            ops.linear_fwd(*a, **k)
+
+    def _lin_bwd(self, *a, **k):
+        if self.gemm_tc:
+            ops.linear_bwd_data_tc(*a, bf16_arena=(self.flat, self.wbf), **k)
+        else:
+            ops.linear_bwd_data(*a, **k)
+
+    def _lin_bww(self, *a, **k):
+        (ops.linear_bwd_weight_tc if self.gemm_tc else ops.linear_bwd_weight)(*a, **k)
 
     # ---------------------------------------------------------------------------------------------- forward
     def _trunk(self, x, acts, M, rows_per_chunk=None, chunk_stride=0):
         r = self.running_mean_std
         nm, ns = (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
-        ops.linear_fwd(x, self.view('W0'), self.view('b0'), acts[0], self.act_id, rows_per_chunk=rows_per_chunk, chunk_stride=chunk_stride,
-                       x_ld=self.S, norm_mean=nm, norm_std=ns, M=M)
+        self._lin_fwd(x, self.view('W0'), self.view('b0'), acts[0], self.act_id, rows_per_chunk=rows_per_chunk, chunk_stride=chunk_stride,
+                      x_ld=self.S, norm_mean=nm, norm_std=ns, M=M)
         for i in range(1, len(self.units)):
-            ops.linear_fwd(acts[i - 1], self.view(f'W{i}'), self.view(f'b{i}'), acts[i], self.act_id, M=M)
+            self._lin_fwd(acts[i - 1], self.view(f'W{i}'), self.view(f'b{i}'), acts[i], self.act_id, M=M)
 
     def get_value(self, states, out):
         """central_value.py:207-229 (eval mode): out[N] = denorm(critic(states))"""
         self._trunk(states, self.r_act, self.N)
+        if self.gemm_tc:        # the fused head: same GEMV arithmetic as training's, de-normalisation in the same launch
+            vm = self.value_mean_std if self.normalize_value else None
+            ops.value_head_fwd(self.r_act[-1], self.view('W_v'), self.view('b_v'), None if vm is None else vm.running_mean,
+                               None if vm is None else vm.running_var, self.normalize_value, out, self.N)
+            return
         ops.linear_fwd(self.r_act[-1], self.view('W_v'), self.view('b_v'), self.r_val, 0, M=self.N)
         if self.normalize_value:
             vm = self.value_mean_std
@@ -199,32 +246,40 @@ class CentralValueNet:
                     ops.moments_update(x, self.S, epm, H, N, r.running_mean, r.running_var, r.count, r.mean_f32, r.std_f32, self.mom_scratch,
                                        self.counters[1:2])
                 self._trunk(x, self.t_act, mb, rows_per_chunk=epm, chunk_stride=N)
-                ops.linear_fwd(self.t_act[-1], self.view('W_v'), self.view('b_v'), self.t_val, 0, M=mb)
-                nb = ops.value_loss(self.t_val, 1, old_values_n[0, e0:], returns_n[0, e0:], None if valid is None else valid[0, e0:], epm, N, mb,
-                                    self.e_clip, self.clip_value, None if valid is None else self.inv_counts[i:i + 1], self.d_val, 1,
-                                    self.loss_partials)
-                rows.append(self.loss_partials[:nb, 0].sum().float())
                 off_w, _ = self.layout['W_v']
                 off_b, _ = self.layout['b_v']
-                ops.linear_bwd_weight(self.d_val, self.t_act[-1], self.part[0, off_w:], self.part[0, off_b:], self.Hl, 1, S_, M=mb, split_stride=P)
-                ops.linear_bwd_data(self.d_val, self.view('W_v'), self.t_act[-1], self.d_act[-1], self.act_id, M=mb)
+                mask, inv = (None, None) if valid is None else (valid[0, e0:], self.inv_counts[i:i + 1])
+                if self.gemm_tc:        # value GEMV + loss + d(a_last) + head gradient in one launch
+                    nb = ops.value_head_loss(self.t_act[-1], self.view('W_v'), self.view('b_v'), old_values_n[0, e0:], returns_n[0, e0:], mask,
+                                             epm, N, mb, self.e_clip, self.clip_value, inv, self.act_id, self.d_act[-1], self.part[0, off_w:],
+                                             self.part[0, off_b:], P, S_, self.loss_partials)
+                    rows.append(self.loss_partials[:nb, 0].sum().float())
+                else:
+                    ops.linear_fwd(self.t_act[-1], self.view('W_v'), self.view('b_v'), self.t_val, 0, M=mb)
+                    nb = ops.value_loss(self.t_val, 1, old_values_n[0, e0:], returns_n[0, e0:], mask, epm, N, mb, self.e_clip, self.clip_value,
+                                        inv, self.d_val, 1, self.loss_partials)
+                    rows.append(self.loss_partials[:nb, 0].sum().float())
+                    ops.linear_bwd_weight(self.d_val, self.t_act[-1], self.part[0, off_w:], self.part[0, off_b:], self.Hl, 1, S_, M=mb,
+                                          split_stride=P)
+                    ops.linear_bwd_data(self.d_val, self.view('W_v'), self.t_act[-1], self.d_act[-1], self.act_id, M=mb)
                 r = self.running_mean_std
                 nm, ns = (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
                 for l in range(len(self.units) - 1, -1, -1):
                     off_w, shp = self.layout[f'W{l}']
                     off_b, _ = self.layout[f'b{l}']
                     if l > 0:
-                        ops.linear_bwd_weight(self.d_act[l], self.t_act[l - 1], self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
-                                              M=mb, split_stride=P)
-                        ops.linear_bwd_data(self.d_act[l], self.view(f'W{l}'), self.t_act[l - 1], self.d_act[l - 1], self.act_id, M=mb)
+                        self._lin_bww(self.d_act[l], self.t_act[l - 1], self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
+                                      M=mb, split_stride=P)
+                        self._lin_bwd(self.d_act[l], self.view(f'W{l}'), self.t_act[l - 1], self.d_act[l - 1], self.act_id, M=mb)
                     else:
-                        ops.linear_bwd_weight(self.d_act[0], x, self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
-                                              rows_per_chunk=epm, chunk_stride=N, x_ld=self.S, norm_mean=nm, norm_std=ns, M=mb, split_stride=P)
+                        self._lin_bww(self.d_act[0], x, self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
+                                      rows_per_chunk=epm, chunk_stride=N, x_ld=self.S, norm_mean=nm, norm_std=ns, M=mb, split_stride=P)
                 ops.reduce_splits(self.part, self.grad, P, S_, split_stride=P)
                 if self.multi_gpu:      # the critic's own flat-gradient exchange, one per minibatch (central_value.py:322-337)
                     dist.all_reduce(self.grad, op=dist.ReduceOp.SUM)
                 ops.adam_step(self.flat, self.grad, self.exp_avg, self.exp_avg_sq, self.opt_state, None, self.opt_cfg, self.adam_stats,
                               self.counters[2:3], n=P)
+                self.refresh_twin()         # on every rank, after the exchange: the next minibatch's GEMMs read the new weights
         self.last_losses = rows
         self.epoch_num += 1
         self.lr, _ = self.scheduler.update(self.lr, 0, self.epoch_num, self.frame, 0)
@@ -260,6 +315,9 @@ class A2CAgentCV(A2CAgent):
                                                  self.max_epochs, self.device_t, multi_gpu=self.multi_gpu, world_size=self.world_size)
         self.central_value_net.writter = self.writer
         self.value_mean_std = self.central_value_net.value_mean_std                        # a2c_continuous.py:72-73
+        if not self.central_value_net.precision_set and self.global_rank == 0:
+            print('b200: central_value_config.mixed_precision not set -> fp32 kernels for the critic; mixed_precision: True in '
+                  'central_value_config runs its layers on the tensor cores (bf16 operands, fp32 accumulate)')
         self._states = None
 
     # ---- env plumbing: keep the privileged view

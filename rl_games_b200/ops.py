@@ -545,3 +545,23 @@ def value_loss(values, value_ld, old_values_n, returns_n, mask, rows_per_chunk, 
                                     float(e_clip), int(clip_value), ptr(inv_count), ptr(d_value), dv_ld, ptr(partials), partials.shape[0],
                                     ctypes.addressof(nb), _stream()), 'value_loss')
     return nb.value
+
+
+VALUE_HEAD_MAX_HL = 4096        # B200RL_VALUE_HEAD_MAX_HL
+
+
+def value_head_loss(a_last, W_v, b_v, old_values_n, returns_n, mask, rows_per_chunk, chunk_stride, M, e_clip, clip_value, inv_count, act_last,
+                    d_alast, dW_part, db_part, split_stride, n_splits, partials, value_out=None):
+    """fused value head of the tensor-core critic (csrc/critic.cu): value GEMV + value_loss + d(a_last) + head gradient split rows"""
+    nb = ctypes.c_int(0)
+    check(lib.b200rl_value_head_loss_f32(ptr(a_last), W_v.numel(), ptr(W_v), ptr(b_v), ptr(old_values_n), ptr(returns_n), ptr(mask),
+                                         rows_per_chunk, chunk_stride, M, float(e_clip), int(clip_value), ptr(inv_count), act_last,
+                                         ptr(d_alast), ptr(value_out), ptr(dW_part), ptr(db_part), split_stride, n_splits, ptr(partials),
+                                         partials.shape[0], ctypes.addressof(nb), _stream()), 'value_head_loss')
+    return nb.value
+
+
+def value_head_fwd(a_last, W_v, b_v, vms_mean, vms_var, normalize_value, values, N):
+    """rollout value of the tensor-core critic: values[N] = denorm(W_v . a_last + b_v) in one launch"""
+    check(lib.b200rl_value_head_fwd_f32(ptr(a_last), W_v.numel(), ptr(W_v), ptr(b_v), ptr(vms_mean), ptr(vms_var), int(normalize_value),
+                                        ptr(values), N, _stream()), 'value_head_fwd')
