@@ -32,10 +32,10 @@ import torch.distributed as dist
 from . import ops
 from .agent import A2CAgent
 from .common import IdentityScheduler, LinearScheduler
-from .model import _RunningStats, check_network_params
+from .model import _RunningStats, FlatArena, adam_opt_state, check_network_params, mlp_backward, mlp_forward
 
 
-class CentralValueNet:
+class CentralValueNet(FlatArena):
     """CentralValueTrain on the fp32 kernels: flat arena [W0 b0 ... W_v b_v] in the reference's parameter order."""
 
     # `CentralValueTrain.model` (central_value.py:44): the reference's Runner wraps it with torch.compile unless the YAML says
@@ -100,18 +100,10 @@ class CentralValueNet:
             raise NotImplementedError(f'central value mixed_precision: the fused value head takes a last layer of at most '
                                       f'{ops.VALUE_HEAD_MAX_HL} units (got {self.Hl})')
         sizes += [('W_v', (1, ins)), ('b_v', (1,))]
-        self.layout, off = OrderedDict(), 0
-        for n, shp in sizes:
-            self.layout[n] = (off, shp)
-            off += int(torch.Size(shp).numel())
-        self.num_params = off
         dev = self.device
-        self.flat = torch.zeros(off, dtype=torch.float32, device=dev)
-        self.exp_avg, self.exp_avg_sq = torch.zeros_like(self.flat), torch.zeros_like(self.flat)
-        for n, (o, shp) in self.layout.items():
-            if n.startswith('W'):
-                bound = 1.0 / float(shp[1]) ** 0.5
-                self.view(n).uniform_(-bound, bound)
+        self._build_arena(sizes, dev)
+        off = self.num_params
+        self._default_init()
         self.running_mean_std = _RunningStats(self.S, dev) if self.normalize_input else None
         self.value_mean_std = _RunningStats(1, dev) if self.normalize_value else None
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)   # noqa: E731
@@ -129,7 +121,7 @@ class CentralValueNet:
         self.inv_counts = f(self.num_minibatches)
         self.mom_scratch = torch.zeros(148 * 4 * 2 * self.S, dtype=torch.float64, device=dev)
         self.counters = torch.zeros(4, dtype=torch.int32, device=dev)
-        self.opt_state = torch.tensor([self.lr, 0.0, 0.0, 0.0], dtype=torch.float64, device=dev)
+        self.opt_state = adam_opt_state(self.lr, 0).to(dev)
         self.adam_stats = f(16)
         # grad_scale = 1/world: the optimiser kernel scales the SUM the all-reduce leaves in self.grad (central_value.py:322-337)
         self.opt_cfg = ops.OptCfg(0.9, 0.999, 1e-8, self.weight_decay, self.grad_norm, 0.0, 1e-6, 1e-2, 1.5,
@@ -138,11 +130,6 @@ class CentralValueNet:
         if self.gemm_tc:
             self.wbf = torch.empty(off, dtype=torch.bfloat16, device=dev)      # bf16 twin of the arena: the GEMMs' weight operands
             self.refresh_twin()
-
-    def view(self, name, arena=None):
-        o, shp = self.layout[name]
-        a = self.flat if arena is None else arena
-        return a[o:o + int(torch.Size(shp).numel())].view(shp)
 
     def param_names(self):
         names = []
@@ -156,31 +143,11 @@ class CentralValueNet:
             out += [self.view(f'W{i}', arena), self.view(f'b{i}', arena)]
         return out + [self.view('W_v', arena), self.view('b_v', arena)]
 
-    def state_dict(self):
-        sd = OrderedDict()
-        if self.normalize_value:
-            sd.update(self.value_mean_std.state_dict('value_mean_std.'))
-        if self.normalize_input:
-            sd.update(self.running_mean_std.state_dict('running_mean_std.'))
-        for n, v in zip(self.param_names(), self._param_views()):
-            sd[n] = v.clone()
-        return sd
-
     def load_state_dict(self, sd, strict=True):
         def strip(k):          # CentralValueTrain.state_dict() prefixes its model's keys with 'model.'; torch.compile adds '_orig_mod.'
             k = k.replace('_orig_mod.', '')
             return k[len('model.'):] if k.startswith('model.') else k
-        sd = {strip(k): v for k, v in sd.items()}
-        with torch.no_grad():
-            for n, v in zip(self.param_names(), self._param_views()):
-                if n in sd:
-                    v.copy_(sd[n].reshape(v.shape))
-                elif strict:
-                    raise KeyError(f'missing key in central value state_dict: {n}')
-            if self.normalize_value and 'value_mean_std.running_mean' in sd:
-                self.value_mean_std.load_state_dict(sd, 'value_mean_std.')
-            if self.normalize_input and 'running_mean_std.running_mean' in sd:
-                self.running_mean_std.load_state_dict(sd, 'running_mean_std.')
+        super().load_state_dict({strip(k): v for k, v in sd.items()}, strict)
         self.refresh_twin()
 
     def refresh_twin(self):
@@ -206,13 +173,13 @@ class CentralValueNet:
         (ops.linear_bwd_weight_tc if self.gemm_tc else ops.linear_bwd_weight)(*a, **k)
 
     # ---------------------------------------------------------------------------------------------- forward
-    def _trunk(self, x, acts, M, rows_per_chunk=None, chunk_stride=0):
+    def _norm(self):
         r = self.running_mean_std
-        nm, ns = (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
-        self._lin_fwd(x, self.view('W0'), self.view('b0'), acts[0], self.act_id, rows_per_chunk=rows_per_chunk, chunk_stride=chunk_stride,
-                      x_ld=self.S, norm_mean=nm, norm_std=ns, M=M)
-        for i in range(1, len(self.units)):
-            self._lin_fwd(acts[i - 1], self.view(f'W{i}'), self.view(f'b{i}'), acts[i], self.act_id, M=M)
+        return (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
+
+    def _trunk(self, x, acts, M, rows_per_chunk=None, chunk_stride=0):
+        mlp_forward(self.layers('', len(self.units)), x, acts, self.act_id, M, self.S, self._norm(), rows_per_chunk, chunk_stride,
+                    lin_fwd=self._lin_fwd)
 
     def get_value(self, states, out):
         """central_value.py:207-229 (eval mode): out[N] = denorm(critic(states))"""
@@ -262,18 +229,8 @@ class CentralValueNet:
                     ops.linear_bwd_weight(self.d_val, self.t_act[-1], self.part[0, off_w:], self.part[0, off_b:], self.Hl, 1, S_, M=mb,
                                           split_stride=P)
                     ops.linear_bwd_data(self.d_val, self.view('W_v'), self.t_act[-1], self.d_act[-1], self.act_id, M=mb)
-                r = self.running_mean_std
-                nm, ns = (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
-                for l in range(len(self.units) - 1, -1, -1):
-                    off_w, shp = self.layout[f'W{l}']
-                    off_b, _ = self.layout[f'b{l}']
-                    if l > 0:
-                        self._lin_bww(self.d_act[l], self.t_act[l - 1], self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
-                                      M=mb, split_stride=P)
-                        self._lin_bwd(self.d_act[l], self.view(f'W{l}'), self.t_act[l - 1], self.d_act[l - 1], self.act_id, M=mb)
-                    else:
-                        self._lin_bww(self.d_act[0], x, self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S_,
-                                      rows_per_chunk=epm, chunk_stride=N, x_ld=self.S, norm_mean=nm, norm_std=ns, M=mb, split_stride=P)
+                mlp_backward(self.layers('', len(self.units)), self.part, x, self.t_act, self.d_act, self.act_id, mb, self.S, self._norm(),
+                             epm, N, lin_bwd=self._lin_bwd, lin_bww=self._lin_bww)
                 ops.reduce_splits(self.part, self.grad, P, S_, split_stride=P)
                 if self.multi_gpu:      # the critic's own flat-gradient exchange, one per minibatch (central_value.py:322-337)
                     dist.all_reduce(self.grad, op=dist.ReduceOp.SUM)
@@ -397,12 +354,6 @@ class A2CAgentCV(A2CAgent):
             cv.load_state_dict(weights['assymetric_vf_nets'])
         osd = weights.get('assymetric_vf_optimizer')
         if osd:
-            step = 0
-            for i, (m, v) in enumerate(zip(cv._param_views(cv.exp_avg), cv._param_views(cv.exp_avg_sq))):
-                if i in osd['state']:
-                    m.copy_(osd['state'][i]['exp_avg'].reshape(m.shape))
-                    v.copy_(osd['state'][i]['exp_avg_sq'].reshape(v.shape))
-                    step = int(float(osd['state'][i]['step']))
-            cv.lr = float(osd['param_groups'][0]['lr'])
-            cv.opt_state.copy_(torch.tensor([cv.lr, float(step), 0.9 ** step if step else 0.0, 0.999 ** step if step else 0.0],
-                                            dtype=torch.float64))
+            lr, step = cv.load_optimizer_state_dict(osd)
+            cv.lr = float(lr)
+            cv.opt_state.copy_(adam_opt_state(cv.lr, step))

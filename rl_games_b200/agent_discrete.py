@@ -5,31 +5,26 @@ DiscreteA2CAgent + common/a2c_common.py:1205-1359 DiscreteA2CBase, models.py:62-
 STATUS: parity-green on a B200 (round 2, ``tests/test_discrete_gpu.py``) against a CPU oracle that is pinned to the reference
 (oracle/ppo_discrete_oracle.py, tests/golden/agent_discrete*.pt).  Everything except the two categorical kernels
 (csrc/discrete.cu) reuses the kernels of the continuous path: linear_fwd / linear_bwd_* / reduce_splits (mlp_simt.cu), gae_fused, prepare_batch, moments_update,
-mask_inv_counts (stats.cu, gae.cu), post_step (rollout.cu), adam_step (adam.cu).
+mask_inv_counts (stats.cu, gae.cu), post_step (rollout.cu), adam_step (adam.cu).  The parameter arena is ``model.FlatArena`` and the
+fp32 trunks are ``model.mlp_forward`` / ``mlp_backward``, shared with the central-value critic; config parsing, the outer train() loop,
+summary scalars, the pooled normaliser sync and checkpoints are ``agent_base.A2CBase``, shared with the continuous agent.
 
 Scope of this first edition: one GPU, eager launches (no CUDA graph), flat Box observations, ``Discrete(K)`` or multi-discrete
 ``Tuple(Discrete(K_j))`` action spaces (K_j <= 64, <= 8 heads), no RNN, no central value.  The scheduler steps once per MINI-EPOCH on the mean KL like the reference
 (a2c_common.py:1265-1272), which costs one host sync per mini-epoch.
 """
-import os
 import time
-from collections import OrderedDict
-from datetime import datetime
 
 import numpy as np
 import torch
 import torch.distributed as dist
 
 from . import ops
-from .agent import _MeterView
-from .model import check_network_params, CompileTolerantModel, _model_call, resolve_device
-from .dist_utils import PackedStatsSync
-from .common import (AdaptiveScheduler, DefaultAlgoObserver, DefaultRewardsShaper, IdentityScheduler, LinearScheduler, create_vec_env,
-                     make_summary_writer)
-from .model import _RunningStats
+from .agent_base import A2CBase
+from .model import FlatArena, _RunningStats, _model_call, adam_opt_state, check_network_params, mlp_backward, mlp_forward
 
 
-class DiscreteModel:
+class DiscreteModel(FlatArena):
     """Flat fp32 parameter arena of A2CBuilder.Network for a discrete space.  Arena order: actor trunk, [critic trunk], fused head
     W_head [1 + K, Hl] (row 0 = value, rows 1.. = logits) and b_head [1 + K]; ``_param_views`` lists the tensors in the reference's
     ``model.parameters()`` order (actor_mlp.*, critic_mlp.*, value.*, logits.*) for state dicts and the index-keyed Adam state."""
@@ -67,30 +62,13 @@ class DiscreteModel:
                 ins = u
         self.Hl = ins
         sizes += [('W_head', (1 + self.K, ins)), ('b_head', (1 + self.K,))]
-        self.layout, off = OrderedDict(), 0
-        for n, shp in sizes:
-            self.layout[n] = (off, shp)
-            off += int(torch.Size(shp).numel())
-        self.num_params = off
-        self.flat = torch.zeros(off, dtype=torch.float32, device=self.device)
-        self.exp_avg = torch.zeros_like(self.flat)
-        self.exp_avg_sq = torch.zeros_like(self.flat)
-        # torch.nn.Linear default weights, zero biases (network_builder.py:332-340 with the 'default' initializer)
-        for n, (o, shp) in self.layout.items():
-            if n.startswith('W'):
-                bound = 1.0 / float(shp[1]) ** 0.5
-                self.view(n).uniform_(-bound, bound)
+        self._build_arena(sizes, self.device)
+        self._default_init()
         self.running_mean_std = _RunningStats(self.D, self.device) if self.normalize_input else None
         self.value_mean_std = _RunningStats(1, self.device) if self.normalize_value else None
 
-    def view(self, name, arena=None):
-        o, shp = self.layout[name]
-        a = self.flat if arena is None else arena
-        return a[o:o + int(torch.Size(shp).numel())].view(shp)
-
     def trunk(self, which):
-        p = 'a' if which == 'actor' or not self.separate else 'c'
-        return [(self.view(f'W{p}{i}'), self.view(f'b{p}{i}')) for i in range(len(self.units))]
+        return self.layers('a' if which == 'actor' or not self.separate else 'c', len(self.units))
 
     def _param_views(self, arena=None):
         out = []
@@ -119,97 +97,24 @@ class DiscreteModel:
             names += [f'a2c_network.logits.{j}.weight', f'a2c_network.logits.{j}.bias']
         return names
 
-    def state_dict(self):
-        sd = OrderedDict()
-        if self.normalize_value:
-            sd.update(self.value_mean_std.state_dict('value_mean_std.'))
-        if self.normalize_input:
-            sd.update(self.running_mean_std.state_dict('running_mean_std.'))
-        for n, v in zip(self.param_names(), self._param_views()):
-            sd[n] = v.clone()
-        return sd
-
-    def load_state_dict(self, sd, strict=True):
-        sd = {k.replace('_orig_mod.', ''): v for k, v in sd.items()}
-        with torch.no_grad():
-            for n, v in zip(self.param_names(), self._param_views()):
-                if n in sd:
-                    v.copy_(sd[n].reshape(v.shape))
-                elif strict:
-                    raise KeyError(f'missing key in state_dict: {n}')
-            if self.normalize_value and 'value_mean_std.running_mean' in sd:
-                self.value_mean_std.load_state_dict(sd, 'value_mean_std.')
-            if self.normalize_input and 'running_mean_std.running_mean' in sd:
-                self.running_mean_std.load_state_dict(sd, 'running_mean_std.')
-
-    def optimizer_state_dict(self, lr, step, weight_decay):
-        state = {i: {'step': torch.tensor(float(step)), 'exp_avg': m.clone(), 'exp_avg_sq': v.clone()}
-                 for i, (m, v) in enumerate(zip(self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq)))}
-        group = {'lr': lr, 'betas': (0.9, 0.999), 'eps': 1e-08, 'weight_decay': weight_decay, 'amsgrad': False, 'maximize': False,
-                 'foreach': None, 'capturable': False, 'differentiable': False, 'fused': True, 'decoupled_weight_decay': False,
-                 'params': list(range(len(state)))}
-        return {'state': state, 'param_groups': [group]}
-
-    def load_optimizer_state_dict(self, osd):
-        st, step = osd.get('state', {}), 0
-        ms, vs = self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq)
-        for i in range(len(ms)):
-            if i in st:
-                ms[i].copy_(st[i]['exp_avg'].reshape(ms[i].shape))
-                vs[i].copy_(st[i]['exp_avg_sq'].reshape(vs[i].shape))
-                step = int(float(st[i]['step']))
-        return (osd['param_groups'][0]['lr'] if osd.get('param_groups') else None), step
-
-
-class DiscreteA2CAgent(CompileTolerantModel):
+class DiscreteA2CAgent(A2CBase):
     def __init__(self, base_name, params):
-        self.config = config = params['config']
-        self.experiment_name = config.get('full_experiment_name') or (config['name'] + datetime.now().strftime("_%d-%H-%M-%S"))
-        config.setdefault('features', {})
-        self.algo_observer = config['features'].get('observer') or DefaultAlgoObserver()
-        self.algo_observer.before_init(base_name, config, self.experiment_name)
-        self.network_params = params['network']
-        # multi-GPU (a2c_common.py:206-220): one process per GPU, actors sharded by rank; the per-minibatch gradient exchange is an NCCL
-        # all-reduce of the flat gradient in front of the Adam kernel (which applies 1/world), the scheduler sees the rank-mean KL
-        self.multi_gpu, self.world_size, self.global_rank, self.local_rank = bool(config.get('multi_gpu', False)), 1, 0, 0
-        if self.multi_gpu:
-            self.local_rank, self.global_rank = int(os.getenv('LOCAL_RANK', '0')), int(os.getenv('RANK', '0'))
-            self.world_size = int(os.getenv('WORLD_SIZE', '1'))
-            config['device'] = 'cuda:' + str(self.local_rank)
-            if not dist.is_initialized():
-                dist.init_process_group('nccl', rank=self.global_rank, world_size=self.world_size, device_id=torch.device(config['device']))
-            if self.global_rank != 0:
-                config['print_stats'] = False
-        self.multi_gpu_sync_stats = config.get('multi_gpu_sync_stats', True)
-        if config.get('multi_gpu_sync_stats_mode', 'pooled') != 'pooled':
-            raise NotImplementedError("multi_gpu_sync_stats_mode: only 'pooled' for the discrete agent")
-        self.ppo_device = config.get('device', 'cuda:0')
-        self._require_cuda()
-        self.device_t = resolve_device(self.ppo_device)          # 'cuda' without an index (configs/ppo_cartpole.yaml) = the current device
-        self.num_actors = config['num_actors']
-        self.env_name = config['env_name']
-        self.env_info = config.get('env_info')
-        if self.env_info is None:
-            self.vec_env = create_vec_env(self.env_name, self.num_actors, **config.get('env_config', {}))
-            self.env_info = self.vec_env.get_env_info()
-        else:
-            self.vec_env = config.get('vec_env', None)
-        if self.env_info.get('agents', 1) != 1 or self.env_info.get('value_size', 1) != 1:
-            raise NotImplementedError('multi-agent envs / value_size > 1')
-        if config.get('central_value_config') is not None:
-            raise NotImplementedError('central_value_config')
+        config = params['config']
         # options of the reference agent that change what a run does and are not built for the discrete path: refuse, never ignore
         for key, bad in (('normalize_rms_advantage', bool(config.get('normalize_rms_advantage', False))),
                          ('epochs_between_resets', config.get('epochs_between_resets', 0) > 0),
                          ('self_play', config.get('self_play_config') is not None or bool(config.get('self_play', False)))):
             if bad:
                 raise NotImplementedError(f'{key} is not built for the discrete B200 agent')
-        self.has_central_value, self.central_value_net = False, None
-        self.num_agents, self.value_size = 1, 1
-        self.observation_space = self.env_info['observation_space']
-        if type(self.observation_space).__name__ == 'Dict' or len(self.observation_space.shape) != 1:
-            raise NotImplementedError('only flat Box observations')
-        self.obs_shape = self.observation_space.shape
+        if config.get('multi_gpu_sync_stats_mode', 'pooled') != 'pooled':
+            raise NotImplementedError("multi_gpu_sync_stats_mode: only 'pooled' for the discrete agent")
+        if config.get('central_value_config') is not None:
+            raise NotImplementedError('central_value_config')
+        # multi-GPU: the per-minibatch gradient exchange is an NCCL all-reduce of the flat gradient in front of the Adam kernel (which
+        # applies 1/world), the scheduler sees the rank-mean KL
+        super().__init__(base_name, params)
+        if self.value_size != 1:
+            raise NotImplementedError('value_size > 1')
         action_space = self.env_info['action_space']
         kind = type(action_space).__name__          # a2c_common.py:1211-1224
         if kind == 'Discrete':
@@ -225,96 +130,12 @@ class DiscreteA2CAgent(CompileTolerantModel):
         if max(self.head_sizes or [self.actions_num]) > 64:
             raise NotImplementedError('more than 64 actions in one discrete head')
         self.use_action_masks = bool(config.get('use_action_masks', False))
-        self.autoreset_mode = self.env_info.get('autoreset_mode', 'same_step')
-        self.mask_autoreset_rows = self.autoreset_mode == 'next_step'
-        self.name = base_name
-        self.ppo = config.get('ppo', True)
-        self.max_epochs = config.get('max_epochs', -1)
-        self.max_frames = max(config.get('max_frames', -1), config.get('max_steps', -1))
-        self.horizon_length = config['horizon_length']
-        self.seq_length = config.get('seq_length', 4)
-        self.normalize_advantage = config['normalize_advantage']
-        if config.get('normalize_rms_advantage', False):
-            raise NotImplementedError('normalize_rms_advantage with the discrete agent')
-        self.normalize_input = config['normalize_input']
-        self.normalize_value = config.get('normalize_value', False)
-        self.critic_coef, self.grad_norm = config['critic_coef'], config['grad_norm']
-        self.gamma, self.tau = config['gamma'], config['tau']
-        self.e_clip, self.clip_value = config['e_clip'], config['clip_value']
-        self.entropy_coef = config['entropy_coef']
-        self.truncate_grads = config.get('truncate_grads', False)
-        self.weight_decay = config.get('weight_decay', 0.0)
-        self.value_bootstrap = config.get('value_bootstrap', True)
-        self.use_smooth_clamp = config.get('use_smooth_clamp', False)
-        self.games_to_track = config.get('games_to_track', 100)
-        self.print_stats = config.get('print_stats', True)
-        self.save_freq, self.save_best_after = config.get('save_frequency', 0), config.get('save_best_after', 100)
-        rs = config['reward_shaper']
-        self.rewards_shaper = rs if not isinstance(rs, dict) else DefaultRewardsShaper(**rs)
-        self.batch_size = self.horizon_length * self.num_actors
-        if 'minibatch_size' not in config and 'minibatch_size_per_env' not in config:
-            raise ValueError("Configuration must include either 'minibatch_size' or 'minibatch_size_per_env'. "
-                             "Neither was found in the provided config.")
-        self.minibatch_size = config.get('minibatch_size', self.num_actors * config.get('minibatch_size_per_env', 0))
-        if self.minibatch_size <= 0 or self.batch_size % self.minibatch_size != 0:
-            raise ValueError(f"'batch_size' ({self.batch_size}) must be divisible by 'minibatch_size' ({self.minibatch_size}).")
-        if self.minibatch_size % self.horizon_length != 0:
-            raise NotImplementedError('minibatch_size must be a multiple of horizon_length (minibatches are whole-env slices of the arena)')
-        self.num_minibatches = self.batch_size // self.minibatch_size
-        self.envs_per_mb = self.minibatch_size // self.horizon_length
-        self.mini_epochs_num = config['mini_epochs']
-        self.last_lr = float(config['learning_rate'])
-        self.is_adaptive_lr = config['lr_schedule'] == 'adaptive'
-        if self.is_adaptive_lr:
-            self.kl_threshold = config['kl_threshold']
-            self.scheduler = AdaptiveScheduler(self.kl_threshold, min_lr=config.get('min_lr', 1e-6), max_lr=config.get('max_lr', 1e-2),
-                                               lr_multiplier=config.get('lr_multiplier', 1.5))
-        elif config['lr_schedule'] == 'linear' and (self.max_epochs != -1 or self.max_frames != -1):
-            use_epochs = self.max_epochs != -1
-            self.scheduler = LinearScheduler(self.last_lr, min_lr=config.get('min_lr', 1e-6),
-                                             max_steps=self.max_epochs if use_epochs else self.max_frames, use_epochs=use_epochs,
-                                             apply_to_entropy=config.get('schedule_entropy', False),
-                                             start_entropy_coef=config.get('entropy_coef'))
-        else:
-            self.scheduler = IdentityScheduler()
-        self.frame = self.epoch_num = self.curr_frames = 0
-        self.mean_rewards = self.last_mean_rewards = -float('inf')
-        self.train_dir = config.get('train_dir', 'runs')
-        self.experiment_dir = os.path.join(self.train_dir, self.experiment_name)
-        self.nn_dir = os.path.join(self.experiment_dir, 'nn')
-        self.summaries_dir = os.path.join(self.experiment_dir, 'summaries')
-        for d in (self.train_dir, self.experiment_dir, self.nn_dir, self.summaries_dir):
-            os.makedirs(d, exist_ok=True)
-        self.writer = make_summary_writer(self.summaries_dir)
         self.model = DiscreteModel(self.network_params, self.obs_shape[0], self.actions_num, self.device_t, self.normalize_input,
                                    self.normalize_value, head_sizes=self.head_sizes)
         self.value_mean_std = self.model.value_mean_std
         self.rng_seed = int(config.get('b200_rng_seed', params.get('seed', 0) or 0))
-        self.is_rnn, self.rnn_states, self.is_tensor_obses = False, None, True
-        self._tensors_ready = False
-        self._meter_cache = None
-        self.obs = None
-        self.game_rewards, self.game_shaped_rewards, self.game_lengths = _MeterView(self, 0), _MeterView(self, 1), _MeterView(self, 2)
+        self.is_tensor_obses = True
         self.algo_observer.after_init(self)
-
-    @property
-    def device(self):
-        return self.ppo_device
-
-    def _require_cuda(self):
-        """no CPU fallback: the kernels are the product (the host-logic test replaces this hook together with every op)"""
-        if not str(self.ppo_device).startswith('cuda'):
-            raise RuntimeError('rl_games_b200 agents run on CUDA only (device=%r): there is no CPU fallback' % self.ppo_device)
-        torch.cuda.set_device(resolve_device(self.ppo_device))
-
-    @staticmethod
-    def _sync():
-        torch.cuda.synchronize()
-
-    def _meter_host(self):
-        if self._meter_cache is None:
-            self._meter_cache = self.meter.cpu().numpy()
-        return self._meter_cache
 
     # =============================================================================== allocation
     def init_tensors(self):
@@ -356,7 +177,7 @@ class DiscreteA2CAgent(CompileTolerantModel):
         self.mom_scratch = torch.zeros(148 * 4 * 2 * D, dtype=torch.float64, device=dev)
         self.post_scratch = torch.zeros(((N + 255) // 256) * 4, dtype=torch.float64, device=dev)
         self.counters = torch.zeros(4, dtype=torch.int32, device=dev)
-        self.opt_state = torch.tensor([self.last_lr, 0.0, 0.0, 0.0], dtype=torch.float64, device=dev)
+        self.opt_state = adam_opt_state(self.last_lr, 0).to(dev)
         self.adam_stats = f(16)
         self.opt_cfg = ops.OptCfg(0.9, 0.999, 1e-8, float(self.weight_decay), float(self.grad_norm), 0.0, 1e-6, 1e-2, 1.5,
                                   1.0 / self.world_size, int(bool(self.truncate_grads)), 0)
@@ -387,13 +208,13 @@ class DiscreteA2CAgent(CompileTolerantModel):
         r = self.model.running_mean_std
         return (r.mean_f32, r.std_f32) if self.normalize_input else (None, None)
 
-    def _trunk(self, layers, x, acts, M, rows_per_chunk=None, chunk_stride=0):
-        nm, ns = self._norm()
+    def _forward(self, x, a_acts, c_acts, head, M, rows_per_chunk=None, chunk_stride=0):
+        """actor trunk, [critic trunk], heads over M rows of x; returns _head_views(head, M)"""
         m = self.model
-        ops.linear_fwd(x, layers[0][0], layers[0][1], acts[0], m.act_id, rows_per_chunk=rows_per_chunk, chunk_stride=chunk_stride,
-                       x_ld=m.D, norm_mean=nm, norm_std=ns, M=M)
-        for i in range(1, len(layers)):
-            ops.linear_fwd(acts[i - 1], layers[i][0], layers[i][1], acts[i], m.act_id, M=M)
+        for which, acts in (('actor', a_acts), ('critic', c_acts))[:1 + m.separate]:
+            mlp_forward(m.trunk(which), x, acts, m.act_id, M, m.D, self._norm(), rows_per_chunk, chunk_stride)
+        self._heads(a_acts[-1], c_acts[-1], head, M)
+        return self._head_views(head, M)
 
     def _heads(self, a_last, c_last, head, M):
         """head[:, 0] = value, head[:, 1:] = logits (one GEMM when the trunk is shared)"""
@@ -438,11 +259,7 @@ class DiscreteA2CAgent(CompileTolerantModel):
             if self.use_action_masks:          # a2c_common.py:995-997
                 masks = self._to_dev(self.vec_env.get_action_masks()).to(torch.uint8).contiguous()
                 self.action_masks[t].copy_(masks)
-            self._trunk(m.trunk('actor'), obs, self.r_a, N)
-            if m.separate:
-                self._trunk(m.trunk('critic'), obs, self.r_c, N)
-            self._heads(self.r_a[-1], self.r_c[-1], self.r_head, N)
-            lg, ld, vl, vld = self._head_views(self.r_head, N)
+            lg, ld, vl, vld = self._forward(obs, self.r_a, self.r_c, self.r_head, N)
             ops.categorical_sample(lg, ld, K, vl, vld, masks, None if u is None else u[t].contiguous(), self.rng_seed, self.rng_epoch, t,
                                    None if vm is None else vm.running_mean, None if vm is None else vm.running_var, self.normalize_value,
                                    self.actions[t], self.neglogpacs[t], self.values[t], self.dones, self.dones_buf[t], self.prev_dones,
@@ -461,11 +278,7 @@ class DiscreteA2CAgent(CompileTolerantModel):
             elif getattr(self.algo_observer, 'wants_infos', False):
                 self.algo_observer.process_infos(infos, None)
         # get_values (a2c_common.py:603-626): the reference's forward samples here too; only the value is used
-        self._trunk(m.trunk('actor'), self.obs, self.r_a, N)
-        if m.separate:
-            self._trunk(m.trunk('critic'), self.obs, self.r_c, N)
-        self._heads(self.r_a[-1], self.r_c[-1], self.r_head, N)
-        lg, ld, vl, vld = self._head_views(self.r_head, N)
+        lg, ld, vl, vld = self._forward(self.obs, self.r_a, self.r_c, self.r_head, N)
         ops.categorical_sample(None, ld, K, vl, vld, None, None, 0, None, 0, None if vm is None else vm.running_mean,
                                None if vm is None else vm.running_var, self.normalize_value, None, None, self.last_values, None, None,
                                None, None, N, values_only=True)
@@ -499,11 +312,7 @@ class DiscreteA2CAgent(CompileTolerantModel):
             r = m.running_mean_std
             ops.moments_update(x, m.D, epm, H, N, r.running_mean, r.running_var, r.count, r.mean_f32, r.std_f32, self.mom_scratch,
                                self.counters[1:2])
-        self._trunk(m.trunk('actor'), x, self.t_a, mb, rows_per_chunk=epm, chunk_stride=N)
-        if m.separate:
-            self._trunk(m.trunk('critic'), x, self.t_c, mb, rows_per_chunk=epm, chunk_stride=N)
-        self._heads(self.t_a[-1], self.t_c[-1], self.t_head, mb)
-        lg, ld, vl, vld = self._head_views(self.t_head, mb)
+        lg, ld, vl, vld = self._forward(x, self.t_a, self.t_c, self.t_head, mb, rows_per_chunk=epm, chunk_stride=N)
         if m.separate:
             d_lg, d_ld, d_vl, d_vld = self._dl_buf(), K, self._dv_buf(), 1
         else:
@@ -519,7 +328,6 @@ class DiscreteA2CAgent(CompileTolerantModel):
         # ---- backward through the heads and the trunk(s): split partial gradients, then one reduction ----
         off_wh, _ = m.layout['W_head']
         off_bh, _ = m.layout['b_head']
-        nm, ns = self._norm()
         if m.separate:
             Hl = m.Hl
             ops.linear_bwd_weight(d_vl, self.t_c[-1], self.part[0, off_wh:], self.part[0, off_bh:], Hl, 1, S, M=mb, split_stride=P)
@@ -527,23 +335,12 @@ class DiscreteA2CAgent(CompileTolerantModel):
             wh = m.view('W_head')
             ops.linear_bwd_data(d_vl, wh[:1], self.t_c[-1], self.d_c[-1], m.act_id, M=mb)
             ops.linear_bwd_data(d_lg, wh[1:], self.t_a[-1], self.d_a[-1], m.act_id, M=mb)
-            trunks = [('a', self.t_a, self.d_a), ('c', self.t_c, self.d_c)]
         else:
             ops.linear_bwd_weight(self.d_head, self.t_a[-1], self.part[0, off_wh:], self.part[0, off_bh:], m.Hl, 1 + K, S, M=mb,
                                   split_stride=P)
             ops.linear_bwd_data(self.d_head, m.view('W_head'), self.t_a[-1], self.d_a[-1], m.act_id, M=mb)
-            trunks = [('a', self.t_a, self.d_a)]
-        for p, acts, dacts in trunks:
-            for l in range(len(m.units) - 1, -1, -1):
-                off_w, shp = m.layout[f'W{p}{l}']
-                off_b, _ = m.layout[f'b{p}{l}']
-                if l > 0:
-                    ops.linear_bwd_weight(dacts[l], acts[l - 1], self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S, M=mb,
-                                          split_stride=P)
-                    ops.linear_bwd_data(dacts[l], m.view(f'W{p}{l}'), acts[l - 1], dacts[l - 1], m.act_id, M=mb)
-                else:
-                    ops.linear_bwd_weight(dacts[0], x, self.part[0, off_w:], self.part[0, off_b:], shp[1], shp[0], S, rows_per_chunk=epm,
-                                          chunk_stride=N, x_ld=m.D, norm_mean=nm, norm_std=ns, M=mb, split_stride=P)
+        for which, acts, dacts in (('actor', self.t_a, self.d_a), ('critic', self.t_c, self.d_c))[:1 + m.separate]:
+            mlp_backward(m.trunk(which), self.part, x, acts, dacts, m.act_id, mb, m.D, self._norm(), epm, N)
         ops.reduce_splits(self.part, self.grad, P, S, split_stride=P)
         if self.multi_gpu:          # a2c_common.py:493-509 (the Adam kernel applies the 1/world scale)
             dist.all_reduce(self.grad, op=dist.ReduceOp.SUM)
@@ -594,154 +391,14 @@ class DiscreteA2CAgent(CompileTolerantModel):
         a_losses, c_losses, entropies = list(st[:, 0]), list(st[:, 1]), list(st[:, 2])
         return step_time, t1 - t0, t2 - t1, t2 - t0, a_losses, c_losses, entropies, kls, lr_used, 1.0
 
-    def update_epoch(self):
-        self.epoch_num += 1
-        return self.epoch_num
-
-    def sync_running_stats(self):
-        """a2c_common.py:782-808, pooled mode: every normaliser's per-epoch moment deltas in ONE packed fp64 all-reduce"""
-        if not self.multi_gpu or not self.multi_gpu_sync_stats:
-            return
-        mods = [(n, r) for n, r in (('obs', self.model.running_mean_std), ('value', self.model.value_mean_std)) if r is not None]
-        if not mods:
-            return
-        if getattr(self, '_stats_sync', None) is None:
-            self._stats_sync = PackedStatsSync([(n, r.count, r.running_mean, r.running_var) for n, r in mods])
-        self._stats_sync.sync(lambda t: dist.all_reduce(t, op=dist.ReduceOp.SUM))
-        for _, r in mods:
-            r.refresh()
-
-    def write_stats(self, total_time, epoch_num, step_time, play_time, update_time, a_losses, c_losses, entropies, kls, last_lr, lr_mul, frame,
-                    scaled_time, scaled_play_time, curr_frames):
-        """a2c_common.py:527-547: the same summary scalars, tag for tag"""
-        w = self.writer
-        mean = lambda xs: float(torch.stack(list(xs)).mean())     # noqa: E731  torch_ext.mean_list
-        w.add_scalar('performance/step_inference_rl_update_fps', curr_frames / scaled_time, frame)
-        w.add_scalar('performance/step_inference_fps', curr_frames / scaled_play_time, frame)
-        w.add_scalar('performance/step_fps', curr_frames / max(step_time, 1e-9), frame)
-        w.add_scalar('performance/rl_update_time', update_time, frame)
-        w.add_scalar('performance/step_inference_time', play_time, frame)
-        w.add_scalar('performance/step_time', step_time, frame)
-        w.add_scalar('losses/a_loss', mean(a_losses), frame)
-        w.add_scalar('losses/c_loss', mean(c_losses), frame)
-        w.add_scalar('losses/entropy', mean(entropies), frame)
-        w.add_scalar('info/last_lr', last_lr * lr_mul, frame)
-        w.add_scalar('info/lr_mul', lr_mul, frame)
-        w.add_scalar('info/e_clip', self.e_clip * lr_mul, frame)
-        w.add_scalar('info/kl', mean(kls), frame)
-        w.add_scalar('info/epochs', epoch_num, frame)
-        self.algo_observer.after_print_stats(frame, epoch_num, total_time)
-
-    def train(self):
-        """DiscreteA2CBase.train (a2c_common.py:1361-1470), single process: frame / epoch accounting, summary scalars, periodic / best /
-        final checkpoints (same file names), score_to_win / max_epochs / max_frames / stop_fn; returns (last_mean_rewards, epoch_num)."""
-        self.init_tensors()
+    # =============================================================================== train loop / checkpoints (agent_base.A2CBase)
+    def _on_train_start(self):
         self.mean_rewards = -float('inf')      # last_mean_rewards (best-ever watermark) is deliberately NOT reset here
-        total_time = 0
-        self.obs = self.env_reset()
-        stop_fn = self.config.get('stop_fn', None)
-        if self.multi_gpu:
-            dist.broadcast(self.model.flat, 0)
-        while True:
-            epoch_num = self.update_epoch()
-            step_time, play_time, update_time, sum_time, a_losses, c_losses, entropies, kls, last_lr, lr_mul = self.train_epoch()
-            total_time += sum_time
-            curr_frames = self.curr_frames * self.world_size if self.multi_gpu else self.curr_frames
-            self.frame += curr_frames
-            should_exit = False
-            frame = self.frame // self.num_agents
-            if self.global_rank != 0:       # rank 0 logs, checkpoints and decides when to stop (a2c_common.py:1391, :1463-1466)
-                t = torch.zeros(1, device=self.device_t)
-                dist.broadcast(t, 0)
-                if bool(t.item()):
-                    return self.last_mean_rewards, epoch_num
-                continue
-            if self.print_stats:
-                print(f'fps step: {curr_frames / max(step_time, 1e-9):.0f} fps step and policy inference: {curr_frames / play_time:.0f} '
-                      f'fps total: {curr_frames / sum_time:.0f} epoch: {epoch_num:.0f}/{self.max_epochs:.0f} frames: {frame:.0f}')
-            if self.writer is not None:
-                self.write_stats(total_time, epoch_num, step_time, play_time, update_time, a_losses, c_losses, entropies, kls, last_lr, lr_mul,
-                                 frame, sum_time, play_time, curr_frames)
-            mean_rewards = None
-            if self.game_rewards.current_size > 0:
-                mean_rewards = self.game_rewards.get_mean()          # float32 array: checkpoint names embed str() of it
-                mean_shaped, mean_lengths = self.game_shaped_rewards.get_mean(), self.game_lengths.get_mean()
-                self.mean_rewards = mean_rewards[0]
-                if self.writer is not None:
-                    for tag, val in (('rewards', mean_rewards[0]), ('shaped_rewards', mean_shaped[0])):
-                        self.writer.add_scalar(tag + '/step', val, frame)
-                        self.writer.add_scalar(tag + '/iter', val, epoch_num)
-                        self.writer.add_scalar(tag + '/time', val, total_time)
-                    self.writer.add_scalar('episode_lengths/step', mean_lengths[0], frame)
-                    self.writer.add_scalar('episode_lengths/iter', mean_lengths[0], epoch_num)
-                    self.writer.add_scalar('episode_lengths/time', mean_lengths[0], total_time)
-                checkpoint_name = self.config['name'] + '_ep_' + str(epoch_num) + '_rew_' + str(mean_rewards[0])
-                if self.save_freq > 0 and epoch_num % self.save_freq == 0:
-                    self.save(os.path.join(self.nn_dir, 'last_' + checkpoint_name))
-                if mean_rewards[0] > self.last_mean_rewards and epoch_num >= self.save_best_after:
-                    print('saving next best rewards: ', mean_rewards)
-                    self.last_mean_rewards = mean_rewards[0]
-                    self.save(os.path.join(self.nn_dir, self.config['name']))
-                    if 'score_to_win' in self.config and self.last_mean_rewards > self.config['score_to_win']:
-                        print('Maximum reward achieved. Network won!')
-                        self.save(os.path.join(self.nn_dir, checkpoint_name))
-                        should_exit = True
-            if epoch_num >= self.max_epochs and self.max_epochs != -1:
-                if self.game_rewards.current_size == 0:
-                    print('WARNING: Max epochs reached before any env terminated at least once')
-                    mean_rewards = -np.inf
-                self.save(os.path.join(self.nn_dir, 'last_' + self.config['name'] + '_ep_' + str(epoch_num)
-                                       + '_rew_' + str(mean_rewards).replace('[', '_').replace(']', '_')))
-                print('MAX EPOCHS NUM!')
-                should_exit = True
-            if self.frame >= self.max_frames and self.max_frames != -1:
-                if self.game_rewards.current_size == 0:
-                    mean_rewards = -np.inf
-                self.save(os.path.join(self.nn_dir, 'last_' + self.config['name'] + '_frame_' + str(self.frame)
-                                       + '_rew_' + str(mean_rewards).replace('[', '_').replace(']', '_')))
-                print('MAX FRAMES NUM!')
-                should_exit = True
-            if not should_exit and stop_fn is not None and stop_fn(self):
-                self.save(os.path.join(self.nn_dir, 'last_' + self.config['name'] + '_custom_stop_ep_' + str(epoch_num)))
-                print('Custom stop callback returned True. Stopping training.')
-                should_exit = True
-            if self.multi_gpu:
-                dist.broadcast(torch.tensor([float(should_exit)], device=self.device_t), 0)
-            if should_exit:
-                return self.last_mean_rewards, epoch_num
 
-    # =============================================================================== weights / checkpoints (a2c_common.py:825-921)
-    def get_weights(self):
-        return {'model': self.model.state_dict()}
+    def _optimizer_lr(self):
+        return float(self.opt_state.cpu()[0])
 
-    def set_weights(self, weights):
-        self.model.load_state_dict(weights['model'])
-
-    def get_full_state_weights(self):
-        self.init_tensors()
-        state = self.get_weights()
-        state['epoch'], state['frame'] = self.epoch_num, self.frame
-        step = float(self.opt_state.cpu()[1])
-        state['optimizer'] = self.model.optimizer_state_dict(float(self.opt_state.cpu()[0]), step, self.weight_decay)      # the optimizer's own lr
-        state['last_mean_rewards'] = self.last_mean_rewards
-        return state
-
-    def set_full_state_weights(self, weights, set_epoch=True):
-        self.init_tensors()
-        self.set_weights(weights)
-        if set_epoch:
-            self.epoch_num, self.frame = weights['epoch'], weights['frame']
-        lr, step = self.model.load_optimizer_state_dict(weights['optimizer'])
-        # a2c_common.py:852-866 restores the optimizer (its lr included) but not last_lr: the restored lr drives the optimiser until the
-        # next scheduler step (end of the first mini-epoch), which continues from this agent's own last_lr
-        opt_lr = float(lr) if lr is not None else self.last_lr
-        self.opt_state.copy_(torch.tensor([opt_lr, float(step), 0.9 ** float(step) if step else 0.0,
-                                           0.999 ** float(step) if step else 0.0], dtype=torch.float64))
-        self.last_mean_rewards = weights.get('last_mean_rewards', -float('inf'))
-
-    def save(self, fn):
-        torch.save(self.get_full_state_weights(), fn + '.pth')
-
-    def restore(self, fn, set_epoch=True):
-        ck = torch.load(fn, map_location=self.device_t, weights_only=False)
-        self.set_full_state_weights(ck, set_epoch=set_epoch)
+    def _restore_optimizer(self, lr, step):
+        # the restored lr drives the optimiser until the next scheduler step (end of the first mini-epoch), which continues from this
+        # agent's own last_lr
+        self.opt_state.copy_(adam_opt_state(float(lr) if lr is not None else self.last_lr, step))

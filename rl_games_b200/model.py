@@ -156,7 +156,127 @@ def _model_call(self, *args, **kwargs):
                               'it has no module-style forward')
 
 
-class B200Model:
+def adam_opt_state(lr, step, slots=4):
+    """the optimiser kernels' state row: lr, step, beta1^step, beta2^step, then zeros up to `slots`"""
+    row = [float(lr), float(step), 0.9 ** float(step) if step else 0.0, 0.999 ** float(step) if step else 0.0]
+    return torch.tensor(row + [0.0] * (slots - 4), dtype=torch.float64)
+
+
+class FlatArena:
+    """Parameters in ONE flat fp32 arena (``flat``) with matching Adam-moment arenas (``exp_avg``, ``exp_avg_sq``), so the optimiser, the
+    gradient all-reduce and the checkpoint code each touch one buffer.  A subclass builds the layout from a ``(name, shape)`` list and
+    defines ``_param_views(arena)``: the tensors in the reference's ``model.parameters()`` order, which the index-keyed Adam state follows.
+    The generic ``state_dict`` / ``load_state_dict`` also need ``param_names()`` (the reference's keys, in the same order)."""
+
+    def _build_arena(self, sizes, device, align=1):
+        """every tensor starts on a multiple of `align` elements; the gaps hold zeros in every arena"""
+        self.layout, off = OrderedDict(), 0
+        for n, shp in sizes:
+            off = (off + align - 1) // align * align
+            self.layout[n] = (off, shp)
+            off += int(torch.Size(shp).numel())
+        self.num_params = off
+        self.flat = torch.zeros(off, dtype=torch.float32, device=device)
+        self.exp_avg = torch.zeros_like(self.flat)
+        self.exp_avg_sq = torch.zeros_like(self.flat)
+
+    def _default_init(self):
+        """torch.nn.Linear default weights on every W* tensor, drawn on the arena's device in layout order; biases stay zero
+        (network_builder.py:332-340 with the 'default' initializer)"""
+        for n, (_, shp) in self.layout.items():
+            if n.startswith('W'):
+                bound = 1.0 / float(shp[1]) ** 0.5
+                self.view(n).uniform_(-bound, bound)
+
+    def view(self, name, arena=None):
+        off, shp = self.layout[name]
+        arena = self.flat if arena is None else arena
+        return arena[off:off + int(torch.Size(shp).numel())].view(shp)
+
+    def layers(self, prefix, n):
+        """[(W, b, offset of W, offset of b)] of the MLP layers W{prefix}{i} / b{prefix}{i}, i < n (see mlp_forward / mlp_backward)"""
+        return [(self.view(f'W{prefix}{i}'), self.view(f'b{prefix}{i}'), self.layout[f'W{prefix}{i}'][0], self.layout[f'b{prefix}{i}'][0])
+                for i in range(n)]
+
+    def state_dict(self):
+        sd = OrderedDict()
+        if self.normalize_value:
+            sd.update(self.value_mean_std.state_dict('value_mean_std.'))
+        if self.normalize_input:
+            sd.update(self.running_mean_std.state_dict('running_mean_std.'))
+        for n, v in zip(self.param_names(), self._param_views(self.flat)):
+            sd[n] = v.clone()
+        return sd
+
+    def load_state_dict(self, sd, strict=True):
+        sd = {k.replace('_orig_mod.', ''): v for k, v in sd.items()}
+        with torch.no_grad():
+            for n, v in zip(self.param_names(), self._param_views(self.flat)):
+                if n in sd:
+                    v.copy_(sd[n].reshape(v.shape))
+                elif strict:
+                    raise KeyError(f'missing key in state_dict: {n}')
+            self._load_normalisers(sd)
+
+    def _load_normalisers(self, sd):
+        if self.normalize_value and 'value_mean_std.running_mean' in sd:
+            self.value_mean_std.load_state_dict(sd, 'value_mean_std.')
+        if self.normalize_input and 'running_mean_std.running_mean' in sd:
+            self.running_mean_std.load_state_dict(sd, 'running_mean_std.')
+
+    def optimizer_state_dict(self, lr, step, weight_decay):
+        """torch.optim.Adam.state_dict() layout (index-keyed, reference parameter order)."""
+        state = {}
+        for i, (m, v) in enumerate(zip(self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq))):
+            state[i] = {'step': torch.tensor(float(step)), 'exp_avg': m.clone(), 'exp_avg_sq': v.clone()}
+        group = {'lr': lr, 'betas': (0.9, 0.999), 'eps': 1e-08, 'weight_decay': weight_decay, 'amsgrad': False,
+                 'maximize': False, 'foreach': None, 'capturable': False, 'differentiable': False, 'fused': True,
+                 'decoupled_weight_decay': False, 'params': list(range(len(state)))}
+        return {'state': state, 'param_groups': [group]}
+
+    def load_optimizer_state_dict(self, osd):
+        """Returns (lr, step)."""
+        st = osd.get('state', {})
+        step = 0
+        ms, vs = self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq)
+        for i in range(len(ms)):
+            if i in st:
+                ms[i].copy_(st[i]['exp_avg'].reshape(ms[i].shape))
+                vs[i].copy_(st[i]['exp_avg_sq'].reshape(vs[i].shape))
+                step = int(float(st[i]['step']))
+        lr = osd['param_groups'][0]['lr'] if osd.get('param_groups') else None
+        return lr, step
+
+
+def mlp_forward(layers, x, acts, act_id, M, x_ld, norm, rows_per_chunk=None, chunk_stride=0, lin_fwd=None):
+    """fp32 MLP trunk over M rows: layer 0 reads the observation rows of x (normalised on the fly by norm = (mean, std) or (None, None),
+    optionally gathered as chunks of rows_per_chunk rows chunk_stride apart), layer i > 0 reads acts[i - 1]; activations go to acts.
+    lin_fwd: the layer GEMM (default ops.linear_fwd, looked up at call time)"""
+    lin_fwd = lin_fwd or ops.linear_fwd
+    lin_fwd(x, layers[0][0], layers[0][1], acts[0], act_id, rows_per_chunk=rows_per_chunk, chunk_stride=chunk_stride, x_ld=x_ld,
+            norm_mean=norm[0], norm_std=norm[1], M=M)
+    for i in range(1, len(layers)):
+        lin_fwd(acts[i - 1], layers[i][0], layers[i][1], acts[i], act_id, M=M)
+
+
+def mlp_backward(layers, part, x, acts, dacts, act_id, M, x_ld, norm, rows_per_chunk, chunk_stride, lin_bwd=None, lin_bww=None):
+    """Backward of mlp_forward, given dacts[-1]: the weight gradients of every layer go to the split-partial rows `part` [splits, P] at the
+    layer's arena offsets, the dgrad chain fills dacts[l - 1]; layer 0's weight gradient re-reads the normalised observation rows of x.
+    lin_bwd / lin_bww: the dgrad / wgrad GEMMs (default ops.linear_bwd_data / ops.linear_bwd_weight, looked up at call time)"""
+    lin_bwd = lin_bwd or ops.linear_bwd_data
+    lin_bww = lin_bww or ops.linear_bwd_weight
+    S, P = part.shape
+    for l in range(len(layers) - 1, -1, -1):
+        W, _, off_w, off_b = layers[l]
+        if l > 0:
+            lin_bww(dacts[l], acts[l - 1], part[0, off_w:], part[0, off_b:], W.shape[1], W.shape[0], S, M=M, split_stride=P)
+            lin_bwd(dacts[l], W, acts[l - 1], dacts[l - 1], act_id, M=M)
+        else:
+            lin_bww(dacts[0], x, part[0, off_w:], part[0, off_b:], W.shape[1], W.shape[0], S, rows_per_chunk=rows_per_chunk,
+                    chunk_stride=chunk_stride, x_ld=x_ld, norm_mean=norm[0], norm_std=norm[1], M=M, split_stride=P)
+
+
+class B200Model(FlatArena):
     __call__ = _model_call
 
     RNN_KEYS = (('a2c_network.rnn.rnn.weight_ih_l0', 'W_ih'), ('a2c_network.rnn.rnn.weight_hh_l0', 'W_hh'),
@@ -229,23 +349,14 @@ class B200Model:
             ins = Hd                     # the heads read the LSTM output
         self.Hl = ins
         sizes += [('W_head', (self.A + 1, ins)), ('b_head', (self.A + 1,))]
-        self.layout = OrderedDict()
-        off = 0
-        for n, shp in sizes:
-            numel = int(torch.Size(shp).numel())
-            # every tensor starts on an 8-element boundary (32 bytes in the fp32 arenas, 16 bytes in the bf16 twin the tensor-core GEMMs
-            # read): weight rows can then be staged with 16-byte loads whatever the action count did to the offsets.  The gaps hold
-            # zeros in every arena (weights, gradients, moments), so norms, Adam and the all-reduce are unaffected; layouts whose tensor
-            # sizes are all multiples of 8 (the BASELINE MLPs with 8 actions) have no gaps at all.
-            off = (off + 7) // 8 * 8
-            self.layout[n] = (off, shp)
-            off += numel
-        self.num_params = off
-        self.flat = torch.zeros(off, dtype=torch.float32, device=self.device)
+        # every tensor starts on an 8-element boundary (32 bytes in the fp32 arenas, 16 bytes in the bf16 twin the tensor-core GEMMs
+        # read): weight rows can then be staged with 16-byte loads whatever the action count did to the offsets.  The gaps hold
+        # zeros in every arena (weights, gradients, moments), so norms, Adam and the all-reduce are unaffected; layouts whose tensor
+        # sizes are all multiples of 8 (the BASELINE MLPs with 8 actions) have no gaps at all.
+        self._build_arena(sizes, self.device, align=8)
+        off = self.num_params
         self.grad = torch.zeros(off, dtype=torch.float32, device=self.device)
-        self.exp_avg = torch.zeros(off, dtype=torch.float32, device=self.device)
-        self.exp_avg_sq = torch.zeros(off, dtype=torch.float32, device=self.device)
-        self.W = [self.view(f'W{i}') for i in range(len(self.units))]
+        self.W =[self.view(f'W{i}') for i in range(len(self.units))]
         self.b = [self.view(f'b{i}') for i in range(len(self.units))]
         self.sigma = self.view('sigma')
         if self.min_sigma > 0:
@@ -289,11 +400,6 @@ class B200Model:
             torch.add(self.sigma_chain, self.min_sigma, out=self.logstd_eff)
             self.sigma_chain.div_(self.logstd_eff)
             self.logstd_eff.log_()
-
-    def view(self, name, arena=None):
-        off, shp = self.layout[name]
-        arena = self.flat if arena is None else arena
-        return arena[off:off + int(torch.Size(shp).numel())].view(shp)
 
     def _init_weights(self, network_params, seed):
         """network_builder.py:326-348: mlp initializer on every Linear weight, zero biases, mu_init on mu.weight,
@@ -447,32 +553,3 @@ class B200Model:
             self.b_head[1:].copy_(sd['a2c_network.mu.bias'])
             self._load_normalisers(sd)
 
-    def _load_normalisers(self, sd):
-        if self.normalize_value and 'value_mean_std.running_mean' in sd:
-            self.value_mean_std.load_state_dict(sd, 'value_mean_std.')
-        if self.normalize_input and 'running_mean_std.running_mean' in sd:
-            self.running_mean_std.load_state_dict(sd, 'running_mean_std.')
-
-    # ------------------------------------------------------------------------------------------- optimizer state
-    def optimizer_state_dict(self, lr, step, weight_decay):
-        """torch.optim.Adam.state_dict() layout (index-keyed, reference parameter order)."""
-        state = {}
-        for i, (m, v) in enumerate(zip(self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq))):
-            state[i] = {'step': torch.tensor(float(step)), 'exp_avg': m.clone(), 'exp_avg_sq': v.clone()}
-        group = {'lr': lr, 'betas': (0.9, 0.999), 'eps': 1e-08, 'weight_decay': weight_decay, 'amsgrad': False,
-                 'maximize': False, 'foreach': None, 'capturable': False, 'differentiable': False, 'fused': True,
-                 'decoupled_weight_decay': False, 'params': list(range(len(state)))}
-        return {'state': state, 'param_groups': [group]}
-
-    def load_optimizer_state_dict(self, osd):
-        """Returns (lr, step)."""
-        st = osd.get('state', {})
-        step = 0
-        ms, vs = self._param_views(self.exp_avg), self._param_views(self.exp_avg_sq)
-        for i in range(len(ms)):
-            if i in st:
-                ms[i].copy_(st[i]['exp_avg'].reshape(ms[i].shape))
-                vs[i].copy_(st[i]['exp_avg_sq'].reshape(vs[i].shape))
-                step = int(float(st[i]['step']))
-        lr = osd['param_groups'][0]['lr'] if osd.get('param_groups') else None
-        return lr, step
